@@ -26,6 +26,12 @@ barrier + synchronize and the slowest rank's device time is used.
 `cpu_baseline`: oracle/_ref/ref_bench (the reference's unmodified mpc_planner.cpp + CppAD, std::thread
             per core; solver inside is the repo's Ipopt stand-in, Ipopt itself is not installed) on all
             host cores, bounded sample; `--impl reference` times the same thing.
+
+`--dump-outputs DIR` writes what the `value` leg computed in its last timed step (rank 0) as float64
+DIR/<name>.npy, one column per problem: the pre-step's coeffs (4) and state (6), the solve's u0 (2),
+pred (3N), obj, status, iters and kkt, and problem = the column's index in the rank's generated input
+sets.  Above DUMP_MAX_PROBLEMS problems a fixed, seeded sample of them is written.  The inputs depend
+only on --batch and --sets, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -52,6 +58,7 @@ FLOP_PER_ITER_N20 = 27879.0  # SURVEY 8d algorithmic flops per interior-point it
 # Algorithmic: 88 B in + ~520 B out per problem = 2.5 MB per launch; the 2.1 MB of results are still in the 126 MB
 # L2 when the kernel ends, so DRAM sees less than the algorithmic bytes -- nothing is re-read.
 NCU_DRAM_BYTES_PER_LAUNCH = 446720
+DUMP_MAX_PROBLEMS = 65536    # 77 float64 values per problem: 40 MB
 
 
 def _ncu_dram_bytes():
@@ -267,6 +274,21 @@ def _pin_to_gpu_numa_node(torch, local):
         return None
 
 
+def dump_outputs(out_dir, sets, B, bufs):
+    """Writes the result buffers of input sets `sets` (name -> per-set device tensors of shape (rows, B) or (B,)) as
+    out_dir/<name>.npy, float64, the sets' problems side by side on the last axis, plus problem.npy."""
+    cols = {"problem": np.concatenate([q * B + np.arange(B) for q in sets]).astype(np.float64)}
+    for name, per_set in bufs.items():
+        cols[name] = np.concatenate([per_set[q].cpu().numpy() for q in sets], axis=-1).astype(np.float64)
+    n = cols["problem"].size
+    if n > DUMP_MAX_PROBLEMS:
+        keep = np.sort(np.random.default_rng(SEED).choice(n, DUMP_MAX_PROBLEMS, replace=False))
+        cols = {k: v[..., keep] for k, v in cols.items()}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, v in cols.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(v))
+
+
 def run_ours(a):
     import torch
     import torch.distributed as dist
@@ -406,6 +428,12 @@ def run_ours(a):
     clocks = sampler.stop() if rank == 0 else None
     ms_total = e0.elapsed_time(e1)
     n_batches = a.steps * NB
+    if a.dump_outputs and rank == 0:
+        # every batch of a step reads one input set and writes that set's result buffers (the same values each time), so
+        # the buffers of the sets the last step used hold what it computed -- until the isolated launches below
+        dump_outputs(a.dump_outputs, sorted({j % R for j in range(jb - NB, jb)}), B,
+                     dict(coeffs=d_coef, state=d_state, u0=d_u0, pred=d_pred, obj=d_obj, status=d_stat, iters=d_it,
+                          kkt=d_kkt))
 
     # converged problems and iterations actually taken in the timed steps (results are deterministic per set)
     conv_steps = 0; iter_steps = 0.0; per_set = {}
@@ -638,7 +666,11 @@ def main():
     ap.add_argument("--e2e-inflight", type=int, default=96, help="ticks in flight over all e2e threads")
     ap.add_argument("--ref-per-core", type=int, default=160)
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed to DIR/<name>.npy (see the module docstring)")
     a = ap.parse_args()
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     if a.warmup < 3:
         a.warmup = 3
     if a.impl == "reference":

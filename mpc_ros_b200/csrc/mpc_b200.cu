@@ -188,8 +188,7 @@ __global__ void __launch_bounds__(128) queue_order_kernel(int batch, const doubl
 // (:365-391) keeps every `step`-th point of the window, beginning with its first, and appends its last point (with
 // path_length / waypoints_dist taken from the parameters instead of the reference's uninitialised members).
 // Closed tracks: indices wrap; at most max_advance points are erased per tick.  One thread per robot.
-// Checked against oracle/mpc_oracle.c (mpc_oracle_cutoff / _downsample), which tests/test_ros_ref.py pins to the
-// reference's own code.
+// Checked against oracle/mpc_oracle.c (mpc_oracle_cutoff / _downsample), the restatement of the reference's code.
 __global__ void window_kernel(int batch, const double *__restrict__ px, const double *__restrict__ py,
                               const int *__restrict__ track_off, const int *__restrict__ track_len,
                               const int *__restrict__ track_id, int *__restrict__ idx_io,

@@ -8,7 +8,7 @@
 //
 //   ref_bench <threads (0 = hardware_concurrency)> <problems per thread> <seed> [offset]
 // Problems: the config-2 generator (bench/problem_gen.cpp) followed by the reference pre-step as restated in
-// oracle/mpc_oracle.c (pinned to driving_state.cpp by tests/test_ros_ref.py).  Prints one JSON object.
+// oracle/mpc_oracle.c (driving_state.cpp restated).  Prints one JSON object.
 #include "mpc_planner.h"
 #include "mpc_oracle.h"
 #include "shim/ip_standin.h"

@@ -7,7 +7,7 @@
 //   * ros_ref_tick_*      : DrivingStateContext + Tracking::mpcComputeVelocityCommands (driving_state.cpp:105-119):
 //                           deceleration (:121-141), findBestPath (:175-271) incl. transform, polyfit, state assembly,
 //                           MPC::Solve, speed clamp
-// They pin oracle/mpc_oracle.c's restatement of those functions to the reference's own code (tests/test_ros_ref.py).
+// With them, oracle/mpc_oracle.c's restatement of those functions can be compared with the reference's own code.
 // (the standard / stub headers first, so that only the reference's own classes are opened up)
 #include <cmath>
 #include <cstring>

@@ -785,8 +785,7 @@ def test_short_and_odd_horizons(oracle):
 # ---------------------------------------------------------------- round 2: windowing, state bounds, large sweeps
 def test_window_kernel_matches_oracle(oracle):
     """SURVEY 8f-2: window_kernel against the oracle's restatement of MPCPlannerROS::getCutOffPlan (:266-291) and
-    downSamplePlan (:365-391) (mpc_oracle_cutoff / _downsample, pinned to the reference's own code by
-    tests/test_ros_ref.py), over several ticks so that the persistent plan index is exercised."""
+    downSamplePlan (:365-391) (mpc_oracle_cutoff / _downsample), over several ticks so that the persistent plan index is exercised."""
     import torch
     from bench import gen_py
     from bench.closed_loop import Fleet
