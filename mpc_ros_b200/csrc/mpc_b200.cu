@@ -331,54 +331,92 @@ __global__ void dfma_kernel(double *out, int iters, int active_lanes, long long 
     if (cycles && threadIdx.x == 0 && blockIdx.x == 0) cycles[0] = t1 - t0;
 }
 
+// ================================================================ solve-kernel specialisations
+// Every compiled solve kernel.  enqueue_solve launches the entry whose key (kind, spt, warm, rate, nc) matches and whose
+// lanes per CTA equal the launch's, else the run-time generic entry (cpb 0) of that key; mpc_b200_create raises the
+// dynamic shared-memory limit of each.
+struct SolveKernel {
+    bool dual;        // nmpc_kernel_dual.cuh: full CTAs as two lane groups out of phase
+    int spt, cpb;     // stages per stage thread; lanes per CTA (0: chosen at run time)
+    bool warm, rate;  // warm start; rate-penalty variant (w_angvel_d / w_accel_d != 0, 44 slots per stage)
+    int nc;           // coefficient rows: 4, or NMPC_MAX_COEFFS for a path polynomial of order 4..7
+    const void *fn;
+};
+#define SK(S, C, W, R, NC) { false, S, C, W, R, NC, (const void *)nmpc::nmpc_solve_kernel<S, C, W, R, NC> }
+#define SK_DUAL(W, R) { true, SPT, (R) ? 28 : 32, W, R, 4, (const void *)nmpc::nmpc_solve_kernel_dual<W, 4, R> }
+static const SolveKernel kSolveKernels[] = {
+    SK(SPT, 0, false, false, 4), SK(SPT, 32, false, false, 4), SK(SPT, 16, false, false, 4), SK(SPT, 8, false, false, 4),
+    SK(SPT, 4, false, false, 4), SK(SPT, 1, false, false, 4),
+    SK(SPT, 6, false, false, 4),                                  // N = 100 (BASELINE config 4)
+    SK(SPT, 0, true, false, 4), SK(SPT, 32, true, false, 4),
+    // 28 lanes: what the 44-slot stages of the rate-penalty variant leave room for at N = 20, the cfg defaults
+    SK(SPT, 0, false, true, 4), SK(SPT, 0, true, true, 4), SK(SPT, 28, false, true, 4), SK(SPT, 28, true, true, 4),
+    // narrow CTAs, one stage per stage thread (the closed loop of BASELINE config 5: 1,024 robots = 8 lanes per CTA)
+    SK(1, 16, false, false, 4), SK(1, 8, false, false, 4), SK(1, 4, false, false, 4), SK(1, 1, false, false, 4),
+    SK(1, 16, true, false, 4), SK(1, 8, true, false, 4), SK(1, 4, true, false, 4), SK(1, 1, true, false, 4),
+    SK_DUAL(false, false), SK_DUAL(true, false), SK_DUAL(false, true), SK_DUAL(true, true),
+    SK(SPT, 0, false, false, NMPC_MAX_COEFFS), SK(SPT, 0, true, false, NMPC_MAX_COEFFS),
+    SK(SPT, 0, false, true, NMPC_MAX_COEFFS), SK(SPT, 0, true, true, NMPC_MAX_COEFFS),
+};
+#undef SK
+#undef SK_DUAL
+
+static const SolveKernel *find_solve_kernel(bool dual, int spt, int pb, bool warm, bool rate, int nc)
+{
+    const SolveKernel *generic = NULL;
+    for (const SolveKernel &k : kSolveKernels) {
+        if (k.dual != dual || k.spt != spt || k.warm != warm || k.rate != rate || k.nc != nc) continue;
+        if (k.cpb == pb) return &k;
+        if (k.cpb == 0) generic = &k;
+    }
+    return generic;
+}
+
 // ================================================================ handle
-// host-buffer results of a tick that is still in flight (mpc_b200_track_submit / _wait)
+// Host-buffer results of a call whose D2H copies are enqueued: the copies that went through the staging area h_out
+// (the destination was not page-locked), moved to their destination by fetch_finish.
 struct Fetch {
-    bool active;
-    bool sliced;           // mpc_b200_track_slice_submit: results went straight into the caller's (page-locked) arrays
-    bool packed;           // mpc_b200_track_packed_submit: one D2H into `io` (or the staging area)
-    void *io; size_t io_off, io_bytes; bool io_pinned;
-    int32_t batch;
-    double *u0, *pred, *obj, *kkt, *cmd, *vel;
-    int32_t *status, *iters;
-    bool pu, pp, po, pk, pc, ps, pi, pv;
+    bool active = false;
+    int n = 0;
+    struct { void *dst; const void *src; size_t bytes; } staged[8];
 };
 
 struct mpc_b200_handle {
     mpc_b200_params params;
-    int device;
-    int max_batch;
-    int num_sms;
-    size_t smem_optin;
-    cudaStream_t stream;
-    cudaEvent_t ev0, ev1;
+    int device = 0;
+    int max_batch = 0;
+    int num_sms = 0;
+    size_t smem_optin = 0;
+    cudaStream_t stream = NULL;
+    cudaEvent_t ev0 = NULL, ev1 = NULL;
     // device scratch
-    double *d_state, *d_coeffs, *d_refv, *d_u0, *d_pred, *d_obj, *d_kkt, *d_warm_out;
-    int *d_status, *d_iters;
-    double *d_wx, *d_wy, *d_pose, *d_cte, *d_vel;
+    double *d_state = NULL, *d_coeffs = NULL, *d_refv = NULL, *d_u0 = NULL, *d_pred = NULL, *d_obj = NULL, *d_kkt = NULL,
+           *d_warm_out = NULL;
+    int *d_status = NULL, *d_iters = NULL;
+    double *d_wx = NULL, *d_wy = NULL, *d_pose = NULL, *d_cte = NULL, *d_vel = NULL;
     // pinned staging
-    double *h_in, *h_out;
-    size_t h_in_bytes, h_out_bytes;
-    int pred_steps;        // horizon the scratch was sized for
-    double last_kernel_s;
-    long long launches;    // API calls that launched work (also drives the queue / order rings)
-    long long kernels;     // kernels launched by this handle
-    long long *d_prof;
-    int opt_dual;
-    int opt_spt1;
-    int *d_queue;          // ring of work-queue heads, one per in-flight launch
-    int *d_order;          // ring of hard-first queue orders (order_ring x max_batch)
-    int order_ring;        // launches that may be in flight on this handle at once (16 .. 1024)
-    int opt_order;         // option: serve the queue hard-first (default on)
-    int max_ctas;          // option: cap on the persistent grid (0 = one CTA per SM)
-    int opt_pb;            // option: problems per CTA (0 = auto)
-    int opt_nc;            // option: rows of the coeffs arrays = polynomial order + 1 (4 .. NMPC_MAX_COEFFS; default 4)
-    double *d_io;          // packed tick buffer (mpc_b200_track_packed_*), allocated on first use
-    size_t d_io_doubles;
-    double *d_warm_stage_in, *d_warm_stage_out;   // device staging of HOST warm-start records, allocated on first use
-    const void *pin_ptr[8]; bool pin_val[8]; int pin_next;   // small cache of cudaPointerGetAttributes answers
-    cudaEvent_t *slot_ev;  // one event per queue / order ring slot: a slot is reused only after its launch has finished
-    Fetch pending;
+    double *h_in = NULL, *h_out = NULL;
+    size_t h_in_bytes = 0, h_out_bytes = 0;
+    int pred_steps = 0;        // horizon the scratch was sized for
+    double last_kernel_s = 0.0;
+    long long launches = 0;    // API calls that launched work (also drives the queue / order rings)
+    long long kernels = 0;     // kernels launched by this handle
+    long long *d_prof = NULL;
+    int opt_dual = 1;
+    int opt_spt1 = 1;
+    int *d_queue = NULL;       // ring of work-queue heads, one per in-flight launch
+    int *d_order = NULL;       // ring of hard-first queue orders (order_ring x max_batch)
+    int order_ring = 0;        // launches that may be in flight on this handle at once (16 .. 1024)
+    int opt_order = 1;         // option: serve the queue hard-first (default on)
+    int max_ctas = 0;          // option: cap on the persistent grid (0 = one CTA per SM)
+    int opt_pb = 0;            // option: problems per CTA (0 = auto)
+    int opt_nc = 4;            // option: rows of the coeffs arrays = polynomial order + 1 (4 .. NMPC_MAX_COEFFS; default 4)
+    double *d_io = NULL;       // packed tick buffer (mpc_b200_track_packed_*), allocated on first use
+    size_t d_io_doubles = 0;
+    double *d_warm_stage_in = NULL, *d_warm_stage_out = NULL;   // device staging of HOST warm-start records, allocated on first use
+    const void *pin_ptr[8] = {}; bool pin_val[8] = {}; int pin_next = 0;   // small cache of cudaPointerGetAttributes answers
+    cudaEvent_t *slot_ev = NULL;   // one event per queue / order ring slot: a slot is reused only after its launch has finished
+    Fetch pending;         // the tick in flight (mpc_b200_track_*_submit / _wait)
     std::string last_err;
 };
 
@@ -418,6 +456,22 @@ static int cuda_fail(mpc_b200_handle *h, cudaError_t e, const char *what)
     return MPC_B200_ERR_CUDA;
 }
 #define CK(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) return cuda_fail(h, e_, #call); } while (0)
+
+// last_kernel_seconds from the events around the last timed launch (once the stream has been synchronised)
+static void read_kernel_time(mpc_b200_handle *h)
+{
+    float ms = 0.f;
+    if (cudaEventElapsedTime(&ms, h->ev0, h->ev1) == cudaSuccess) h->last_kernel_s = 1e-3 * ms; else cudaGetLastError();
+}
+
+// End of a device-only entry point that launched one kernel: count it; without a caller stream, return once it has run.
+static int finish_device_call(mpc_b200_handle *h, cudaStream_t st, void *stream_v)
+{
+    CK(cudaGetLastError());
+    h->launches++; h->kernels++;
+    if (!stream_v) CK(cudaStreamSynchronize(st));
+    return MPC_B200_OK;
+}
 
 static void free_scratch(mpc_b200_handle *h)
 {
@@ -534,14 +588,7 @@ int mpc_b200_create(mpc_b200_handle **out, const mpc_b200_params *p, int32_t max
     }
     mpc_b200_handle *h = new (std::nothrow) mpc_b200_handle();
     if (!h) return MPC_B200_ERR_NOMEM;
-    h->params = *p; h->device = device; h->max_batch = max_batch; h->last_kernel_s = 0.0; h->launches = 0; h->kernels = 0;
-    h->d_state = h->d_coeffs = h->d_refv = h->d_u0 = h->d_pred = h->d_obj = h->d_kkt = h->d_warm_out = NULL;
-    h->d_status = h->d_iters = NULL; h->d_wx = h->d_wy = h->d_pose = h->d_cte = h->d_vel = NULL; h->h_in = h->h_out = NULL;
-    h->stream = NULL; h->ev0 = h->ev1 = NULL; h->d_prof = NULL; h->d_queue = NULL; h->max_ctas = 0; h->opt_pb = 0; h->opt_nc = 4; h->d_order = NULL; h->opt_order = 1; h->opt_dual = 1; h->opt_spt1 = 1;
-    h->d_io = NULL; h->d_io_doubles = 0; h->d_warm_stage_in = h->d_warm_stage_out = NULL; h->slot_ev = NULL; h->order_ring = 0;
-    for (int i = 0; i < 8; i++) { h->pin_ptr[i] = NULL; h->pin_val[i] = false; }
-    h->pin_next = 0;
-    h->pending = Fetch();
+    h->params = *p; h->device = device; h->max_batch = max_batch;
     cudaError_t e = cudaSetDevice(device);
     if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking);
     if (e == cudaSuccess) e = cudaEventCreate(&h->ev0);
@@ -551,25 +598,8 @@ int mpc_b200_create(mpc_b200_handle **out, const mpc_b200_params *p, int32_t max
     if (e == cudaSuccess) e = cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, device);
     if (e != cudaSuccess) { cudaGetLastError(); delete h; return MPC_B200_ERR_CUDA; }
     h->num_sms = sms; h->smem_optin = (size_t)optin;
-#define SET_SMEM(K) if (e == cudaSuccess) e = cudaFuncSetAttribute(K, cudaFuncAttributeMaxDynamicSharedMemorySize, optin)
-    SET_SMEM((nmpc::nmpc_solve_kernel<SPT, 0, false, false>)); SET_SMEM((nmpc::nmpc_solve_kernel<SPT, 32, false, false>));
-    SET_SMEM((nmpc::nmpc_solve_kernel<SPT, 16, false, false>)); SET_SMEM((nmpc::nmpc_solve_kernel<SPT, 8, false, false>));
-    SET_SMEM((nmpc::nmpc_solve_kernel<SPT, 4, false, false>)); SET_SMEM((nmpc::nmpc_solve_kernel<SPT, 1, false, false>));
-    SET_SMEM((nmpc::nmpc_solve_kernel<SPT, 0, true, false>)); SET_SMEM((nmpc::nmpc_solve_kernel<SPT, 32, true, false>));
-    // rate-penalty variant (w_angvel_d / w_accel_d != 0): 44 slots per stage, lanes per CTA chosen at run time
-    SET_SMEM((nmpc::nmpc_solve_kernel<SPT, 0, false, true>)); SET_SMEM((nmpc::nmpc_solve_kernel<SPT, 0, true, true>));
-    SET_SMEM((nmpc::nmpc_solve_kernel<SPT, 28, false, true>)); SET_SMEM((nmpc::nmpc_solve_kernel<SPT, 28, true, true>));
-    SET_SMEM((nmpc::nmpc_solve_kernel<SPT, 6, false, false>));
-    SET_SMEM((nmpc::nmpc_solve_kernel<1, 16, false, false>)); SET_SMEM((nmpc::nmpc_solve_kernel<1, 8, false, false>));
-    SET_SMEM((nmpc::nmpc_solve_kernel<1, 4, false, false>)); SET_SMEM((nmpc::nmpc_solve_kernel<1, 1, false, false>));
-    SET_SMEM((nmpc::nmpc_solve_kernel<1, 16, true, false>)); SET_SMEM((nmpc::nmpc_solve_kernel<1, 8, true, false>));
-    SET_SMEM((nmpc::nmpc_solve_kernel<1, 4, true, false>)); SET_SMEM((nmpc::nmpc_solve_kernel<1, 1, true, false>));
-    SET_SMEM((nmpc::nmpc_solve_kernel_dual<false>)); SET_SMEM((nmpc::nmpc_solve_kernel_dual<true>));
-    SET_SMEM((nmpc::nmpc_solve_kernel_dual<false, 4, true>)); SET_SMEM((nmpc::nmpc_solve_kernel_dual<true, 4, true>));
-    // path polynomial of order 4..7
-    SET_SMEM((nmpc::nmpc_solve_kernel<SPT, 0, false, false, NMPC_MAX_COEFFS>)); SET_SMEM((nmpc::nmpc_solve_kernel<SPT, 0, true, false, NMPC_MAX_COEFFS>));
-    SET_SMEM((nmpc::nmpc_solve_kernel<SPT, 0, false, true, NMPC_MAX_COEFFS>)); SET_SMEM((nmpc::nmpc_solve_kernel<SPT, 0, true, true, NMPC_MAX_COEFFS>));
-#undef SET_SMEM
+    for (const SolveKernel &k : kSolveKernels)
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(k.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, optin);
     if (e != cudaSuccess) { cudaGetLastError(); delete h; return MPC_B200_ERR_CUDA; }
     rc = alloc_scratch(h, h->params.mpc_steps);
     if (rc == MPC_B200_OK) rc = alloc_rings(h);
@@ -730,8 +760,14 @@ static int enqueue_solve(mpc_b200_handle *h, int32_t batch, const double *d_stat
                      spt1_threads <= NMPC_MAX_THREADS(1, a.PB)) ? 1 : SPT;
     a.prm.grp = spt;
     const int NG = (N + spt - 1) / spt;
-    const int stage_threads = ((NG * a.PB + 31) / 32) * 32;
-    const int threads = NMPC_CTRL_THREADS + stage_threads;
+    // full CTAs: two lane groups out of phase, one stage per stage thread and group
+    const bool dual = h->opt_dual && a.ncoef <= 4 && a.PB == (rate ? 28 : 32) && N > 10 && N <= NMPC_DUAL_MAX_N;
+    const SolveKernel *kern = find_solve_kernel(dual, spt, a.PB, a.warm_in != NULL, rate, a.ncoef > 4 ? NMPC_MAX_COEFFS : 4);
+    if (!kern) {
+        h->last_err = "no compiled solve kernel for this configuration";
+        return MPC_B200_ERR_UNSUPPORTED;
+    }
+    const int threads = NMPC_CTRL_THREADS + ((dual ? 16 * N : NG * a.PB) + 31) / 32 * 32;
     // persistent grid: at most one CTA per SM (or the max_ctas option); lanes refill from the queue
     int grid = (batch + a.PB - 1) / a.PB;
     const int cap = h->max_ctas > 0 ? h->max_ctas : h->num_sms;
@@ -761,83 +797,38 @@ static int enqueue_solve(mpc_b200_handle *h, int32_t batch, const double *d_stat
         CK(cudaMemsetAsync(a.queue, 0, sizeof(int), st));
     }
     if (timed) CK(cudaEventRecord(h->ev0, st));
-    if (h->opt_dual && a.ncoef <= 4 && a.PB == (rate ? 28 : 32) && N > 10 && N <= NMPC_DUAL_MAX_N) {
-        // full CTAs: two lane groups out of phase, one stage per stage thread and group
-        const int dthreads = NMPC_CTRL_THREADS + ((16 * N + 31) / 32) * 32;
-        if (rate && a.warm_in) nmpc::nmpc_solve_kernel_dual<true, 4, true><<<grid, dthreads, smem, st>>>(a);
-        else if (rate) nmpc::nmpc_solve_kernel_dual<false, 4, true><<<grid, dthreads, smem, st>>>(a);
-        else if (a.warm_in) nmpc::nmpc_solve_kernel_dual<true><<<grid, dthreads, smem, st>>>(a);
-        else nmpc::nmpc_solve_kernel_dual<false><<<grid, dthreads, smem, st>>>(a);
-    } else if (a.ncoef > 4) {
-        if (rate && a.warm_in) nmpc::nmpc_solve_kernel<SPT, 0, true, true, NMPC_MAX_COEFFS><<<grid, threads, smem, st>>>(a);
-        else if (rate) nmpc::nmpc_solve_kernel<SPT, 0, false, true, NMPC_MAX_COEFFS><<<grid, threads, smem, st>>>(a);
-        else if (a.warm_in) nmpc::nmpc_solve_kernel<SPT, 0, true, false, NMPC_MAX_COEFFS><<<grid, threads, smem, st>>>(a);
-        else nmpc::nmpc_solve_kernel<SPT, 0, false, false, NMPC_MAX_COEFFS><<<grid, threads, smem, st>>>(a);
-    } else if (rate) {
-        // (28 lanes: what the 44-slot stages of the rate-penalty variant leave room for at N = 20, the cfg defaults)
-        if (a.warm_in) {
-            if (a.PB == 28) nmpc::nmpc_solve_kernel<SPT, 28, true, true><<<grid, threads, smem, st>>>(a);
-            else nmpc::nmpc_solve_kernel<SPT, 0, true, true><<<grid, threads, smem, st>>>(a);
-        } else {
-            if (a.PB == 28) nmpc::nmpc_solve_kernel<SPT, 28, false, true><<<grid, threads, smem, st>>>(a);
-            else nmpc::nmpc_solve_kernel<SPT, 0, false, true><<<grid, threads, smem, st>>>(a);
-        }
-    } else if (a.warm_in && spt != 1) {
-        if (a.PB == 32) nmpc::nmpc_solve_kernel<SPT, 32, true, false><<<grid, threads, smem, st>>>(a);
-        else nmpc::nmpc_solve_kernel<SPT, 0, true, false><<<grid, threads, smem, st>>>(a);
-    } else if (spt == 1 && a.warm_in) switch (a.PB) {      // (the closed loop of BASELINE config 5: 1,024 robots = 8 lanes per CTA)
-        case 16: nmpc::nmpc_solve_kernel<1, 16, true, false><<<grid, threads, smem, st>>>(a); break;
-        case 8: nmpc::nmpc_solve_kernel<1, 8, true, false><<<grid, threads, smem, st>>>(a); break;
-        case 4: nmpc::nmpc_solve_kernel<1, 4, true, false><<<grid, threads, smem, st>>>(a); break;
-        default: nmpc::nmpc_solve_kernel<1, 1, true, false><<<grid, threads, smem, st>>>(a); break;
-    } else if (spt == 1) switch (a.PB) {
-        case 16: nmpc::nmpc_solve_kernel<1, 16, false, false><<<grid, threads, smem, st>>>(a); break;
-        case 8: nmpc::nmpc_solve_kernel<1, 8, false, false><<<grid, threads, smem, st>>>(a); break;
-        case 4: nmpc::nmpc_solve_kernel<1, 4, false, false><<<grid, threads, smem, st>>>(a); break;
-        default: nmpc::nmpc_solve_kernel<1, 1, false, false><<<grid, threads, smem, st>>>(a); break;
-    } else switch (a.PB) {
-        case 32: nmpc::nmpc_solve_kernel<SPT, 32, false, false><<<grid, threads, smem, st>>>(a); break;
-        case 16: nmpc::nmpc_solve_kernel<SPT, 16, false, false><<<grid, threads, smem, st>>>(a); break;
-        case 8: nmpc::nmpc_solve_kernel<SPT, 8, false, false><<<grid, threads, smem, st>>>(a); break;
-        case 6: nmpc::nmpc_solve_kernel<SPT, 6, false, false><<<grid, threads, smem, st>>>(a); break;   // N = 100 (BASELINE config 4)
-        case 4: nmpc::nmpc_solve_kernel<SPT, 4, false, false><<<grid, threads, smem, st>>>(a); break;
-        case 1: nmpc::nmpc_solve_kernel<SPT, 1, false, false><<<grid, threads, smem, st>>>(a); break;
-        default: nmpc::nmpc_solve_kernel<SPT, 0, false, false><<<grid, threads, smem, st>>>(a); break;
-    }
-    CK(cudaGetLastError());
+    void *args[] = {&a};
+    CK(cudaLaunchKernel(kern->fn, dim3(grid), dim3(threads), args, smem, st));
     if (timed) CK(cudaEventRecord(h->ev1, st));
     CK(cudaEventRecord(h->slot_ev[slot], st));
     h->launches++; h->kernels++;
     return MPC_B200_OK;
 }
 
-// D2H of the solve results into host buffers (direct when they are page-locked): the copies are enqueued
-// by fetch_enqueue; fetch_finish synchronises and moves what went through the staging buffer.
-
-static void fetch_layout(mpc_b200_handle *h, size_t B, double **u0, double **pred, double **obj, double **kkt, double **cmd,
-                         double **vel, int **status, int **iters)
+// D2H of results into host buffers: straight into `dst` when it is page-locked, else into the staging area at `stage`,
+// from where fetch_finish moves it once the stream has run.
+static cudaError_t fetch_copy(Fetch &f, void *dst, void *stage, const void *src, size_t bytes, bool pinned, cudaStream_t st)
 {
-    const size_t N = (size_t)h->params.mpc_steps;
-    double *ho = h->h_out;
-    *u0 = ho; *pred = ho + 2 * B; *obj = *pred + 3 * N * B; *kkt = *obj + B; *cmd = *kkt + B; *vel = *cmd + 2 * B;
-    *status = reinterpret_cast<int *>(*vel + 3 * B); *iters = *status + B;
+    if (!pinned) f.staged[f.n++] = {dst, stage, bytes};
+    return cudaMemcpyAsync(pinned ? dst : stage, src, bytes, cudaMemcpyDeviceToHost, st);
 }
 
-static int fetch_enqueue(mpc_b200_handle *h, Fetch &f, cudaStream_t st)
+// the solve results (and a tick's cmd / vel) from the handle's scratch; h_out: u0 pred obj kkt cmd vel status iters
+static int fetch_enqueue(mpc_b200_handle *h, Fetch &f, int32_t batch, double *u0, double *pred, double *obj, double *kkt,
+                         int32_t *status, int32_t *iters, double *cmd, double *vel, cudaStream_t st)
 {
-    const size_t B = (size_t)f.batch, N = (size_t)h->params.mpc_steps;
-    double *ho_u0, *ho_pred, *ho_obj, *ho_kkt, *ho_cmd, *ho_vel; int *ho_status, *ho_iters;
-    fetch_layout(h, B, &ho_u0, &ho_pred, &ho_obj, &ho_kkt, &ho_cmd, &ho_vel, &ho_status, &ho_iters);
-    f.pu = is_pinned_cached(h, f.u0); f.pp = is_pinned_cached(h, f.pred); f.po = is_pinned_cached(h, f.obj); f.pk = is_pinned_cached(h, f.kkt);
-    f.ps = is_pinned_cached(h, f.status); f.pi = is_pinned_cached(h, f.iters); f.pc = is_pinned_cached(h, f.cmd); f.pv = is_pinned_cached(h, f.vel);
-    CK(cudaMemcpyAsync(f.pu ? f.u0 : ho_u0, h->d_u0, sizeof(double) * 2 * B, cudaMemcpyDeviceToHost, st));
-    CK(cudaMemcpyAsync(f.pp ? f.pred : ho_pred, h->d_pred, sizeof(double) * 3 * N * B, cudaMemcpyDeviceToHost, st));
-    if (f.obj) CK(cudaMemcpyAsync(f.po ? f.obj : ho_obj, h->d_obj, sizeof(double) * B, cudaMemcpyDeviceToHost, st));
-    if (f.kkt) CK(cudaMemcpyAsync(f.pk ? f.kkt : ho_kkt, h->d_kkt, sizeof(double) * B, cudaMemcpyDeviceToHost, st));
-    if (f.status) CK(cudaMemcpyAsync(f.ps ? f.status : ho_status, h->d_status, sizeof(int) * B, cudaMemcpyDeviceToHost, st));
-    if (f.iters) CK(cudaMemcpyAsync(f.pi ? f.iters : ho_iters, h->d_iters, sizeof(int) * B, cudaMemcpyDeviceToHost, st));
-    if (f.cmd) CK(cudaMemcpyAsync(f.pc ? f.cmd : ho_cmd, h->d_cte, sizeof(double) * 2 * B, cudaMemcpyDeviceToHost, st));
-    if (f.vel) CK(cudaMemcpyAsync(f.pv ? f.vel : ho_vel, h->d_vel, sizeof(double) * 3 * B, cudaMemcpyDeviceToHost, st));
+    const size_t B = (size_t)batch, N = (size_t)h->params.mpc_steps;
+    double *ho = h->h_out, *ho_obj = ho + (2 + 3 * N) * B, *ho_cmd = ho_obj + 2 * B, *ho_vel = ho_cmd + 2 * B;
+    int *ho_status = reinterpret_cast<int *>(ho_vel + 3 * B);
+    f = Fetch();
+    CK(fetch_copy(f, u0, ho, h->d_u0, sizeof(double) * 2 * B, is_pinned_cached(h, u0), st));
+    CK(fetch_copy(f, pred, ho + 2 * B, h->d_pred, sizeof(double) * 3 * N * B, is_pinned_cached(h, pred), st));
+    if (obj) CK(fetch_copy(f, obj, ho_obj, h->d_obj, sizeof(double) * B, is_pinned_cached(h, obj), st));
+    if (kkt) CK(fetch_copy(f, kkt, ho_obj + B, h->d_kkt, sizeof(double) * B, is_pinned_cached(h, kkt), st));
+    if (status) CK(fetch_copy(f, status, ho_status, h->d_status, sizeof(int) * B, is_pinned_cached(h, status), st));
+    if (iters) CK(fetch_copy(f, iters, ho_status + B, h->d_iters, sizeof(int) * B, is_pinned_cached(h, iters), st));
+    if (cmd) CK(fetch_copy(f, cmd, ho_cmd, h->d_cte, sizeof(double) * 2 * B, is_pinned_cached(h, cmd), st));
+    if (vel) CK(fetch_copy(f, vel, ho_vel, h->d_vel, sizeof(double) * 3 * B, is_pinned_cached(h, vel), st));
     f.active = true;
     return MPC_B200_OK;
 }
@@ -846,35 +837,9 @@ static int fetch_finish(mpc_b200_handle *h, Fetch &f, cudaStream_t st)
 {
     if (!f.active) return MPC_B200_OK;
     f.active = false;
-    if (f.sliced) {
-        f.sliced = false;
-        CK(cudaStreamSynchronize(st));
-        float ms = 0.f;
-        if (cudaEventElapsedTime(&ms, h->ev0, h->ev1) == cudaSuccess) h->last_kernel_s = 1e-3 * ms; else cudaGetLastError();
-        return MPC_B200_OK;
-    }
-    if (f.packed) {
-        f.packed = false;
-        CK(cudaStreamSynchronize(st));
-        if (!f.io_pinned) memcpy((char *)f.io + f.io_off, h->h_out, f.io_bytes);
-        float ms = 0.f;
-        if (cudaEventElapsedTime(&ms, h->ev0, h->ev1) == cudaSuccess) h->last_kernel_s = 1e-3 * ms; else cudaGetLastError();
-        return MPC_B200_OK;
-    }
-    const size_t B = (size_t)f.batch, N = (size_t)h->params.mpc_steps;
-    double *ho_u0, *ho_pred, *ho_obj, *ho_kkt, *ho_cmd, *ho_vel; int *ho_status, *ho_iters;
-    fetch_layout(h, B, &ho_u0, &ho_pred, &ho_obj, &ho_kkt, &ho_cmd, &ho_vel, &ho_status, &ho_iters);
     CK(cudaStreamSynchronize(st));
-    if (!f.pu) memcpy(f.u0, ho_u0, sizeof(double) * 2 * B);
-    if (!f.pp) memcpy(f.pred, ho_pred, sizeof(double) * 3 * N * B);
-    if (f.obj && !f.po) memcpy(f.obj, ho_obj, sizeof(double) * B);
-    if (f.kkt && !f.pk) memcpy(f.kkt, ho_kkt, sizeof(double) * B);
-    if (f.status && !f.ps) memcpy(f.status, ho_status, sizeof(int) * B);
-    if (f.iters && !f.pi) memcpy(f.iters, ho_iters, sizeof(int) * B);
-    if (f.cmd && !f.pc) memcpy(f.cmd, ho_cmd, sizeof(double) * 2 * B);
-    if (f.vel && !f.pv) memcpy(f.vel, ho_vel, sizeof(double) * 3 * B);
-    float ms = 0.f;
-    if (cudaEventElapsedTime(&ms, h->ev0, h->ev1) == cudaSuccess) h->last_kernel_s = 1e-3 * ms; else cudaGetLastError();
+    for (int i = 0; i < f.n; i++) memcpy(f.staged[i].dst, f.staged[i].src, f.staged[i].bytes);
+    read_kernel_time(h);
     return MPC_B200_OK;
 }
 
@@ -941,17 +906,34 @@ int mpc_b200_solve_batch(mpc_b200_handle *h, int32_t batch,
     }
 
     if (!dev_out) {
-        Fetch f = {};
-        f.batch = batch; f.u0 = u0; f.pred = pred; f.obj = obj; f.kkt = kkt_res; f.status = status; f.iters = iters;
-        rc = fetch_enqueue(h, f, st);
+        Fetch f;
+        rc = fetch_enqueue(h, f, batch, u0, pred, obj, kkt_res, status, iters, NULL, NULL, st);
         if (rc != MPC_B200_OK) return rc;
         return fetch_finish(h, f, st);
     }
     if (!(dev_in && stream_v)) {
         CK(cudaStreamSynchronize(st));
-        float ms = 0.f;
-        if (cudaEventElapsedTime(&ms, h->ev0, h->ev1) == cudaSuccess) h->last_kernel_s = 1e-3 * ms; else cudaGetLastError();
+        read_kernel_time(h);
     }
+    return MPC_B200_OK;
+}
+
+// One control tick on `st` once its inputs are on the device: pre-step into the handle's state / coeffs scratch, solve,
+// post-step (cmd, and w / throttle back into vel for the next tick's delay compensation).
+static int enqueue_tick(mpc_b200_handle *h, cudaStream_t st, int32_t batch, int32_t M, const double *d_wx, const double *d_wy,
+                        const double *d_pose, double *d_vel, const double *d_refv, double *d_u0, double *d_pred,
+                        double *d_obj, int32_t *d_status, int32_t *d_iters, double *d_kkt, double *d_cmd)
+{
+    launch_prestep(h->opt_nc, st, batch, M, d_wx, d_wy, d_pose, h->d_coeffs, NULL, d_vel, h->d_state, h->params.delay_mode,
+                   h->params.dt);
+    CK(cudaGetLastError());
+    h->kernels++;
+    const int rc = enqueue_solve(h, batch, h->d_state, h->d_coeffs, d_refv, NULL, d_u0, d_pred, d_obj, d_status, d_iters, d_kkt,
+                                 NULL, st);
+    if (rc != MPC_B200_OK) return rc;
+    poststep_kernel<<<(batch + 127) / 128, 128, 0, st>>>(batch, d_u0, d_vel, d_refv, h->params.ref_vel, h->params.dt, d_cmd);
+    CK(cudaGetLastError());
+    h->kernels++;
     return MPC_B200_OK;
 }
 
@@ -983,22 +965,11 @@ int mpc_b200_track_submit(mpc_b200_handle *h, int32_t batch, int32_t M,
     CK(cudaMemcpyAsync(h->d_pose, sp, sizeof(double) * 3 * B, cudaMemcpyHostToDevice, st));
     CK(cudaMemcpyAsync(h->d_vel, sv, sizeof(double) * 3 * B, cudaMemcpyHostToDevice, st));
     if (ref_vel) CK(cudaMemcpyAsync(h->d_refv, sr, sizeof(double) * B, cudaMemcpyHostToDevice, st));
-    launch_prestep(h->opt_nc, st, batch, M, h->d_wx, h->d_wy, h->d_pose, h->d_coeffs, NULL, h->d_vel, h->d_state,
-                   h->params.delay_mode, h->params.dt);
-    CK(cudaGetLastError());
-    h->kernels++;
-    int rc = enqueue_solve(h, batch, h->d_state, h->d_coeffs, ref_vel ? h->d_refv : NULL, NULL, h->d_u0, h->d_pred, h->d_obj,
-                           h->d_status, h->d_iters, h->d_kkt, NULL, st);
+    const int rc = enqueue_tick(h, st, batch, M, h->d_wx, h->d_wy, h->d_pose, h->d_vel, ref_vel ? h->d_refv : NULL, h->d_u0,
+                                h->d_pred, h->d_obj, h->d_status, h->d_iters, h->d_kkt, h->d_cte);
     if (rc != MPC_B200_OK) return rc;
-    poststep_kernel<<<(batch + 127) / 128, 128, 0, st>>>(batch, h->d_u0, h->d_vel, ref_vel ? h->d_refv : NULL, h->params.ref_vel,
-                                                          h->params.dt, h->d_cte);
-    CK(cudaGetLastError());
-    h->kernels++;
     // previous w / throttle for the next tick's delay compensation go back into the caller's vel buffer
-    Fetch &f = h->pending;
-    f.batch = batch; f.u0 = u0; f.pred = pred; f.obj = obj; f.kkt = kkt_res; f.status = status; f.iters = iters;
-    f.cmd = cmd_out; f.vel = vel_inout;
-    return fetch_enqueue(h, f, st);
+    return fetch_enqueue(h, h->pending, batch, u0, pred, obj, kkt_res, status, iters, cmd_out, vel_inout, st);
 }
 
 // ---- packed tick: ONE caller buffer, one H2D and one D2H copy per tick
@@ -1068,20 +1039,12 @@ int mpc_b200_track_packed_submit(mpc_b200_handle *h, int32_t batch, int32_t M, i
     double *d_wx = d + off[0], *d_wy = d + off[1], *d_pose = d + off[2], *d_refv = off[3] >= 0 ? d + off[3] : NULL, *d_vel = d + off[4];
     double *d_u0 = d + off[5], *d_pred = d + off[6], *d_cmd = d + off[7], *d_obj = d + off[8], *d_kkt = d + off[9];
     int *d_status = reinterpret_cast<int *>(d + off[10]), *d_iters = reinterpret_cast<int *>(d + off[11]);
-    launch_prestep(h->opt_nc, st, batch, M, d_wx, d_wy, d_pose, h->d_coeffs, NULL, d_vel, h->d_state, h->params.delay_mode,
-                   h->params.dt);
-    CK(cudaGetLastError());
-    h->kernels++;
-    int rc = enqueue_solve(h, batch, h->d_state, h->d_coeffs, d_refv, NULL, d_u0, d_pred, d_obj, d_status, d_iters, d_kkt, NULL, st);
+    const int rc = enqueue_tick(h, st, batch, M, d_wx, d_wy, d_pose, d_vel, d_refv, d_u0, d_pred, d_obj, d_status, d_iters, d_kkt,
+                                d_cmd);
     if (rc != MPC_B200_OK) return rc;
-    poststep_kernel<<<(batch + 127) / 128, 128, 0, st>>>(batch, d_u0, d_vel, d_refv, h->params.ref_vel, h->params.dt, d_cmd);
-    CK(cudaGetLastError());
-    h->kernels++;
     Fetch &f = h->pending;
     f = Fetch();
-    f.packed = true; f.io = io; f.io_off = out_off; f.io_bytes = out_bytes; f.io_pinned = pinned; f.batch = batch;
-    CK(cudaMemcpyAsync(pinned ? (void *)((char *)io + out_off) : (void *)h->h_out, (const char *)d + out_off, out_bytes,
-                       cudaMemcpyDeviceToHost, st));
+    CK(fetch_copy(f, (char *)io + out_off, h->h_out, (const char *)d + out_off, out_bytes, pinned, st));
     f.active = true;
     return MPC_B200_OK;
 }
@@ -1115,17 +1078,9 @@ int mpc_b200_track_slice_submit(mpc_b200_handle *h, int32_t ld, int32_t offset, 
 #define D2H2(dst, src, rows) CK(cudaMemcpy2DAsync((dst) + offset, hp, src, dp, w, (size_t)(rows), cudaMemcpyDeviceToHost, st))
     H2D2(h->d_wx, wx, M); H2D2(h->d_wy, wy, M); H2D2(h->d_pose, pose, 3); H2D2(h->d_vel, vel_inout, 3);
     if (ref_vel) H2D2(h->d_refv, ref_vel, 1);
-    launch_prestep(h->opt_nc, st, batch, M, h->d_wx, h->d_wy, h->d_pose, h->d_coeffs, NULL, h->d_vel, h->d_state,
-                   h->params.delay_mode, h->params.dt);
-    CK(cudaGetLastError());
-    h->kernels++;
-    int rc = enqueue_solve(h, batch, h->d_state, h->d_coeffs, ref_vel ? h->d_refv : NULL, NULL, h->d_u0, h->d_pred, h->d_obj,
-                           h->d_status, h->d_iters, h->d_kkt, NULL, st);
+    const int rc = enqueue_tick(h, st, batch, M, h->d_wx, h->d_wy, h->d_pose, h->d_vel, ref_vel ? h->d_refv : NULL, h->d_u0,
+                                h->d_pred, h->d_obj, h->d_status, h->d_iters, h->d_kkt, h->d_cte);
     if (rc != MPC_B200_OK) return rc;
-    poststep_kernel<<<(batch + 127) / 128, 128, 0, st>>>(batch, h->d_u0, h->d_vel, ref_vel ? h->d_refv : NULL, h->params.ref_vel,
-                                                          h->params.dt, h->d_cte);
-    CK(cudaGetLastError());
-    h->kernels++;
     D2H2(u0, h->d_u0, 2); D2H2(pred, h->d_pred, 3 * N); D2H2(vel_inout, h->d_vel, 3);
     if (cmd_out) D2H2(cmd_out, h->d_cte, 2);
     if (obj) D2H2(obj, h->d_obj, 1);
@@ -1134,9 +1089,8 @@ int mpc_b200_track_slice_submit(mpc_b200_handle *h, int32_t ld, int32_t offset, 
     if (iters) CK(cudaMemcpyAsync(iters + offset, h->d_iters, sizeof(int32_t) * B, cudaMemcpyDeviceToHost, st));
 #undef H2D2
 #undef D2H2
-    Fetch &f = h->pending;
-    f = Fetch();
-    f.sliced = true; f.batch = batch; f.active = true;
+    h->pending = Fetch();      // nothing staged: the copies go straight into the caller's arrays
+    h->pending.active = true;
     return MPC_B200_OK;
 }
 
@@ -1171,54 +1125,65 @@ int mpc_b200_track_batch(mpc_b200_handle *h, int32_t batch, int32_t M,
     return mpc_b200_track_wait(h);
 }
 
+// The pre-step kernel with one of its optional outputs: cte / etheta (cte_eth_out), or the solver's initial state
+// (state_out, from vel).  Inputs and outputs are each either all device or all host memory; host arrays are staged.
+static int prestep_call(mpc_b200_handle *h, int32_t batch, int32_t M, const double *wx, const double *wy, const double *pose,
+                        const double *vel, double *coeffs_out, double *cte_eth_out, double *state_out, void *stream_v)
+{
+    if (M < h->opt_nc || M > MAX_WAYPOINTS) return MPC_B200_ERR_INVALID;   // polyfit asserts order <= M-1 (driving_state.cpp:286)
+    if (batch == 0) return MPC_B200_OK;
+    CK(cudaSetDevice(h->device));
+    const size_t B = (size_t)batch, nc = (size_t)h->opt_nc;
+    cudaStream_t st = stream_v ? (cudaStream_t)stream_v : h->stream;
+    const bool dev_in = is_device_ptr(wx), dev_out = is_device_ptr(coeffs_out);
+    if (is_device_ptr(wy) != dev_in || is_device_ptr(pose) != dev_in || (vel && is_device_ptr(vel) != dev_in))
+        return MPC_B200_ERR_INVALID;
+    if ((cte_eth_out && is_device_ptr(cte_eth_out) != dev_out) || (state_out && is_device_ptr(state_out) != dev_out))
+        return MPC_B200_ERR_INVALID;
+    const double *dwx = wx, *dwy = wy, *dpose = pose, *dvel = vel;
+    if (!dev_in) {
+        double *hi = h->h_in;
+        memcpy(hi, wx, sizeof(double) * M * B);
+        memcpy(hi + (size_t)M * B, wy, sizeof(double) * M * B);
+        memcpy(hi + 2 * (size_t)M * B, pose, sizeof(double) * 3 * B);
+        if (vel) memcpy(hi + 2 * (size_t)M * B + 3 * B, vel, sizeof(double) * 3 * B);
+        CK(cudaMemcpyAsync(h->d_wx, hi, sizeof(double) * M * B, cudaMemcpyHostToDevice, st));
+        CK(cudaMemcpyAsync(h->d_wy, hi + (size_t)M * B, sizeof(double) * M * B, cudaMemcpyHostToDevice, st));
+        CK(cudaMemcpyAsync(h->d_pose, hi + 2 * (size_t)M * B, sizeof(double) * 3 * B, cudaMemcpyHostToDevice, st));
+        if (vel) CK(cudaMemcpyAsync(h->d_vel, hi + 2 * (size_t)M * B + 3 * B, sizeof(double) * 3 * B, cudaMemcpyHostToDevice, st));
+        dwx = h->d_wx; dwy = h->d_wy; dpose = h->d_pose; dvel = vel ? h->d_vel : NULL;
+    }
+    double *dco = dev_out ? coeffs_out : h->d_coeffs;
+    double *dce = cte_eth_out ? (dev_out ? cte_eth_out : h->d_cte) : NULL;
+    double *dso = state_out ? (dev_out ? state_out : h->d_state) : NULL;
+    CK(cudaEventRecord(h->ev0, st));
+    launch_prestep(h->opt_nc, st, batch, M, dwx, dwy, dpose, dco, dce, dvel, dso, h->params.delay_mode, h->params.dt);
+    CK(cudaGetLastError());
+    CK(cudaEventRecord(h->ev1, st));
+    h->launches++; h->kernels++;
+    if (!dev_out) {
+        // h_out: coeffs, then cte / etheta or the state
+        Fetch f;
+        CK(fetch_copy(f, coeffs_out, h->h_out, dco, sizeof(double) * nc * B, false, st));
+        if (dce) CK(fetch_copy(f, cte_eth_out, h->h_out + nc * B, dce, sizeof(double) * 2 * B, false, st));
+        if (dso) CK(fetch_copy(f, state_out, h->h_out + nc * B, dso, sizeof(double) * 6 * B, false, st));
+        f.active = true;
+        return fetch_finish(h, f, st);
+    }
+    if (!(dev_in && stream_v)) {
+        CK(cudaStreamSynchronize(st));
+        read_kernel_time(h);
+    }
+    return MPC_B200_OK;
+}
+
 int mpc_b200_polyfit_batch(mpc_b200_handle *h, int32_t batch, int32_t M,
                            const double *wx, const double *wy, const double *pose,
                            double *coeffs_out, double *cte_etheta_out, void *stream_v)
 {
     NvtxRange nv("mpc_b200_polyfit_batch");
     if (!h || batch < 0 || batch > h->max_batch || !wx || !wy || !pose || !coeffs_out) return MPC_B200_ERR_INVALID;
-    if (M < h->opt_nc || M > MAX_WAYPOINTS) return MPC_B200_ERR_INVALID;   // polyfit asserts order <= M-1 (driving_state.cpp:286)
-    if (batch == 0) return MPC_B200_OK;
-    CK(cudaSetDevice(h->device));
-    const size_t B = (size_t)batch;
-    cudaStream_t st = stream_v ? (cudaStream_t)stream_v : h->stream;
-    const bool dev_in = is_device_ptr(wx), dev_out = is_device_ptr(coeffs_out);
-    if (is_device_ptr(wy) != dev_in || is_device_ptr(pose) != dev_in) return MPC_B200_ERR_INVALID;
-    if (cte_etheta_out && is_device_ptr(cte_etheta_out) != dev_out) return MPC_B200_ERR_INVALID;
-    const double *dwx = wx, *dwy = wy, *dpose = pose;
-    if (!dev_in) {
-        double *hi = h->h_in;
-        memcpy(hi, wx, sizeof(double) * M * B);
-        memcpy(hi + (size_t)M * B, wy, sizeof(double) * M * B);
-        memcpy(hi + 2 * (size_t)M * B, pose, sizeof(double) * 3 * B);
-        CK(cudaMemcpyAsync(h->d_wx, hi, sizeof(double) * M * B, cudaMemcpyHostToDevice, st));
-        CK(cudaMemcpyAsync(h->d_wy, hi + (size_t)M * B, sizeof(double) * M * B, cudaMemcpyHostToDevice, st));
-        CK(cudaMemcpyAsync(h->d_pose, hi + 2 * (size_t)M * B, sizeof(double) * 3 * B, cudaMemcpyHostToDevice, st));
-        dwx = h->d_wx; dwy = h->d_wy; dpose = h->d_pose;
-    }
-    double *dco = dev_out ? coeffs_out : h->d_coeffs;
-    double *dce = cte_etheta_out ? (dev_out ? cte_etheta_out : h->d_cte) : NULL;
-    CK(cudaEventRecord(h->ev0, st));
-    launch_prestep(h->opt_nc, st, batch, M, dwx, dwy, dpose, dco, dce, NULL, NULL, 0, 0.0);
-    CK(cudaGetLastError());
-    CK(cudaEventRecord(h->ev1, st));
-    h->launches++; h->kernels++;
-    if (!dev_out) {
-        double *ho = h->h_out;
-        const size_t nc = (size_t)h->opt_nc;
-        CK(cudaMemcpyAsync(ho, dco, sizeof(double) * nc * B, cudaMemcpyDeviceToHost, st));
-        if (dce) CK(cudaMemcpyAsync(ho + nc * B, dce, sizeof(double) * 2 * B, cudaMemcpyDeviceToHost, st));
-        CK(cudaStreamSynchronize(st));
-        memcpy(coeffs_out, ho, sizeof(double) * nc * B);
-        if (dce) memcpy(cte_etheta_out, ho + nc * B, sizeof(double) * 2 * B);
-    } else if (!(dev_in && stream_v)) {
-        CK(cudaStreamSynchronize(st));
-    }
-    if (!(dev_in && dev_out && stream_v)) {
-        float ms = 0.f;
-        if (cudaEventElapsedTime(&ms, h->ev0, h->ev1) == cudaSuccess) h->last_kernel_s = 1e-3 * ms; else cudaGetLastError();
-    }
-    return MPC_B200_OK;
+    return prestep_call(h, batch, M, wx, wy, pose, NULL, coeffs_out, cte_etheta_out, NULL, stream_v);
 }
 
 int mpc_b200_prestep_batch(mpc_b200_handle *h, int32_t batch, int32_t M,
@@ -1228,50 +1193,7 @@ int mpc_b200_prestep_batch(mpc_b200_handle *h, int32_t batch, int32_t M,
     NvtxRange nv("mpc_b200_prestep_batch");
     if (!h || batch < 0 || batch > h->max_batch || !wx || !wy || !pose || !vel || !coeffs_out || !state_out)
         return MPC_B200_ERR_INVALID;
-    if (M < h->opt_nc || M > MAX_WAYPOINTS) return MPC_B200_ERR_INVALID;
-    if (batch == 0) return MPC_B200_OK;
-    CK(cudaSetDevice(h->device));
-    const size_t B = (size_t)batch;
-    cudaStream_t st = stream_v ? (cudaStream_t)stream_v : h->stream;
-    const bool dev_in = is_device_ptr(wx), dev_out = is_device_ptr(coeffs_out);
-    if (is_device_ptr(wy) != dev_in || is_device_ptr(pose) != dev_in || is_device_ptr(vel) != dev_in) return MPC_B200_ERR_INVALID;
-    if (is_device_ptr(state_out) != dev_out) return MPC_B200_ERR_INVALID;
-    const double *dwx = wx, *dwy = wy, *dpose = pose, *dvel = vel;
-    if (!dev_in) {
-        double *hi = h->h_in;
-        memcpy(hi, wx, sizeof(double) * M * B);
-        memcpy(hi + (size_t)M * B, wy, sizeof(double) * M * B);
-        memcpy(hi + 2 * (size_t)M * B, pose, sizeof(double) * 3 * B);
-        memcpy(hi + 2 * (size_t)M * B + 3 * B, vel, sizeof(double) * 3 * B);
-        CK(cudaMemcpyAsync(h->d_wx, hi, sizeof(double) * M * B, cudaMemcpyHostToDevice, st));
-        CK(cudaMemcpyAsync(h->d_wy, hi + (size_t)M * B, sizeof(double) * M * B, cudaMemcpyHostToDevice, st));
-        CK(cudaMemcpyAsync(h->d_pose, hi + 2 * (size_t)M * B, sizeof(double) * 3 * B, cudaMemcpyHostToDevice, st));
-        CK(cudaMemcpyAsync(h->d_vel, hi + 2 * (size_t)M * B + 3 * B, sizeof(double) * 3 * B, cudaMemcpyHostToDevice, st));
-        dwx = h->d_wx; dwy = h->d_wy; dpose = h->d_pose; dvel = h->d_vel;
-    }
-    double *dco = dev_out ? coeffs_out : h->d_coeffs;
-    double *dso = dev_out ? state_out : h->d_state;
-    CK(cudaEventRecord(h->ev0, st));
-    launch_prestep(h->opt_nc, st, batch, M, dwx, dwy, dpose, dco, NULL, dvel, dso, h->params.delay_mode, h->params.dt);
-    CK(cudaGetLastError());
-    CK(cudaEventRecord(h->ev1, st));
-    h->launches++; h->kernels++;
-    if (!dev_out) {
-        double *ho = h->h_out;
-        const size_t nc = (size_t)h->opt_nc;
-        CK(cudaMemcpyAsync(ho, dco, sizeof(double) * nc * B, cudaMemcpyDeviceToHost, st));
-        CK(cudaMemcpyAsync(ho + nc * B, dso, sizeof(double) * 6 * B, cudaMemcpyDeviceToHost, st));
-        CK(cudaStreamSynchronize(st));
-        memcpy(coeffs_out, ho, sizeof(double) * nc * B);
-        memcpy(state_out, ho + nc * B, sizeof(double) * 6 * B);
-    } else if (!(dev_in && stream_v)) {
-        CK(cudaStreamSynchronize(st));
-    }
-    if (!(dev_in && dev_out && stream_v)) {
-        float ms = 0.f;
-        if (cudaEventElapsedTime(&ms, h->ev0, h->ev1) == cudaSuccess) h->last_kernel_s = 1e-3 * ms; else cudaGetLastError();
-    }
-    return MPC_B200_OK;
+    return prestep_call(h, batch, M, wx, wy, pose, vel, coeffs_out, NULL, state_out, stream_v);
 }
 
 int mpc_b200_window_batch(mpc_b200_handle *h, int32_t batch, const double *path_x, const double *path_y,
@@ -1292,10 +1214,7 @@ int mpc_b200_window_batch(mpc_b200_handle *h, int32_t batch, const double *path_
     cudaStream_t st = stream_v ? (cudaStream_t)stream_v : h->stream;
     window_kernel<<<(batch + 127) / 128, 128, 0, st>>>(batch, path_x, path_y, track_off, track_len, track_id, idx_inout,
                                                         pose, win, step, 64, wx_out, wy_out);
-    CK(cudaGetLastError());
-    h->launches++; h->kernels++;
-    if (!stream_v) CK(cudaStreamSynchronize(st));
-    return MPC_B200_OK;
+    return finish_device_call(h, st, stream_v);
 }
 
 int mpc_b200_poststep_batch(mpc_b200_handle *h, int32_t batch, const double *u0, double *vel_inout,
@@ -1308,10 +1227,7 @@ int mpc_b200_poststep_batch(mpc_b200_handle *h, int32_t batch, const double *u0,
     CK(cudaSetDevice(h->device));
     cudaStream_t st = stream_v ? (cudaStream_t)stream_v : h->stream;
     poststep_kernel<<<(batch + 127) / 128, 128, 0, st>>>(batch, u0, vel_inout, ref_vel, h->params.ref_vel, h->params.dt, cmd_out);
-    CK(cudaGetLastError());
-    h->launches++; h->kernels++;
-    if (!stream_v) CK(cudaStreamSynchronize(st));
-    return MPC_B200_OK;
+    return finish_device_call(h, st, stream_v);
 }
 
 int mpc_b200_decel_batch(mpc_b200_handle *h, int32_t batch, const double *pose, const double *goal, const double *vel,
@@ -1325,10 +1241,7 @@ int mpc_b200_decel_batch(mpc_b200_handle *h, int32_t batch, const double *pose, 
     cudaStream_t st = stream_v ? (cudaStream_t)stream_v : h->stream;
     const double thr = h->params.max_throttle < 0.1 ? 0.1 : h->params.max_throttle;      // driving_state.cpp:63
     decel_kernel<<<(batch + 127) / 128, 128, 0, st>>>(batch, pose, goal, vel, thr, h->params.max_speed, min_speed, ref_vel_inout);
-    CK(cudaGetLastError());
-    h->launches++; h->kernels++;
-    if (!stream_v) CK(cudaStreamSynchronize(st));
-    return MPC_B200_OK;
+    return finish_device_call(h, st, stream_v);
 }
 
 int mpc_b200_plant_step_batch(mpc_b200_handle *h, int32_t batch, const double *cmd, double *pose_inout, double *vel_inout,
@@ -1340,10 +1253,7 @@ int mpc_b200_plant_step_batch(mpc_b200_handle *h, int32_t batch, const double *c
     CK(cudaSetDevice(h->device));
     cudaStream_t st = stream_v ? (cudaStream_t)stream_v : h->stream;
     plant_kernel<<<(batch + 127) / 128, 128, 0, st>>>(batch, cmd, pose_inout, vel_inout, h->params.dt);
-    CK(cudaGetLastError());
-    h->launches++; h->kernels++;
-    if (!stream_v) CK(cudaStreamSynchronize(st));
-    return MPC_B200_OK;
+    return finish_device_call(h, st, stream_v);
 }
 
 int mpc_b200_num_waypoints(const mpc_b200_params *p)
@@ -1364,10 +1274,7 @@ int mpc_b200_warm_shift(mpc_b200_handle *h, int32_t batch, const double *warm_pr
     CK(cudaSetDevice(h->device));
     cudaStream_t st = stream_v ? (cudaStream_t)stream_v : h->stream;
     warm_shift_kernel<<<(batch + 127) / 128, 128, 0, st>>>(batch, h->params.mpc_steps, warm_prev, warm_next);
-    CK(cudaGetLastError());
-    h->launches++; h->kernels++;
-    if (!stream_v) CK(cudaStreamSynchronize(st));
-    return MPC_B200_OK;
+    return finish_device_call(h, st, stream_v);
 }
 
 double mpc_b200_measure_fp64_peak(int32_t device, int32_t iters)
