@@ -573,7 +573,7 @@ const char *mpc_b200_strerror(int code)
 
 const char *mpc_b200_last_cuda_error(const mpc_b200_handle *h) { return h ? h->last_err.c_str() : ""; }
 
-int32_t mpc_b200_warm_size(int32_t N) { return (8 * N - 2) + 6 * N + 4 * (N - 1); }
+int32_t mpc_b200_warm_size(int32_t N) { return (int32_t)nmpc::warm_size(N); }
 
 int mpc_b200_create(mpc_b200_handle **out, const mpc_b200_params *p, int32_t max_batch, int32_t device)
 {

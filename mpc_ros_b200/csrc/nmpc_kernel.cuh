@@ -26,27 +26,6 @@
 
 namespace nmpc {
 
-struct SolveArgs {
-    Params prm;
-    int PB;
-    int batch;
-    int ncoef;              // rows of coeffs: 4 (cubic) .. NMPC_MAX_COEFFS
-    const double *state;    // 6 x batch
-    const double *coeffs;   // ncoef x batch
-    const double *ref_vel;  // batch or NULL
-    double *u0;             // 2 x batch
-    double *pred;           // 3N x batch
-    double *obj;            // batch or NULL
-    int *status;            // batch or NULL
-    int *iters;             // batch or NULL
-    double *kkt;            // batch or NULL
-    double *warm_out;       // warm_size x batch or NULL
-    const double *warm_in;  // warm_size x batch or NULL (cold start)
-    int *queue;             // work-queue head (zeroed by the host before the launch)
-    const int *order;       // queue position -> problem index (hard-first order) or NULL (identity)
-    long long *prof;        // NMPC_PROFILE builds only: per-phase cycle counters of CTA 0
-};
-
 #ifdef NMPC_PROFILE
 #define PROF_DECL long long prof_t = clock64(), prof_acc[12] = {0,0,0,0,0,0,0,0,0,0,0,0}
 #define PROF_MARK(i) do { long long t_ = clock64(); prof_acc[i] += t_ - prof_t; prof_t = t_; } while (0)
@@ -117,35 +96,10 @@ __device__ __forceinline__ void control_loop(const SolveArgs &a, const SM &sm, c
             if (fin) {
                 int nidx = nb + __popc(m & ((1u << wl) - 1u));
                 if (nidx >= batch) nidx = -1;
-                else {
-                    if (a.order) nidx = a.order[nidx];
-                    for (int i = 0; i < 6; i++) sm.P(PS_NX0 + i, p) = a.state[(size_t)i * batch + nidx];
-                    for (int i = 0; i < 4; i++) sm.P(PS_NX6 + i, p) = a.coeffs[(size_t)i * batch + nidx];
-                    if (NC > 4)
-                        for (int i = 4; i < NC; i++)
-                            sm.P(PS_NXC4 + (i - 4), p) = i < a.ncoef ? a.coeffs[(size_t)i * batch + nidx] : 0.0;
-                    sm.P(PS_NX10, p) = a.ref_vel ? a.ref_vel[nidx] : prm.ref_vel;
-                }
+                else if (a.order) nidx = a.order[nidx];
                 sm.I(PI_NEXT, p) = nidx;
-                if (nidx >= 0) {
-                    double s6[6];
-                    for (int i = 0; i < 6; i++) s6[i] = sm.P(PS_NX0 + i, p);
-                    ctrl_init(prm, sm, c, p, s6, sm.P(PS_NX10, p));
-                    if (WARM) {
-                        sm.P(PS_MU, p) = prm.warm_mu; sm.P(PS_MU_STEP, p) = prm.warm_mu;
-                        sm.P(PS_TAU, p) = fmax2(NMPC_TAU_MIN, 1.0 - prm.warm_mu);
-                        const size_t offl = (size_t)(8 * N - 2);
-                        for (int i = 0; i < 6; i++)
-                            sm.P(PS_L0X + i, p) = sm.P(PS_SF, p) * a.warm_in[(offl + (size_t)i * N) * batch + nidx];
-                        sm.I(PI_MODE, p) = MODE_ROLLOUT;
-                        sm.I(PI_FLAGS, p) |= FL_WARM;
-                    } else {
-                        sm.I(PI_MODE, p) = MODE_NEWTON;
-                        sm.I(PI_FLAGS, p) |= FL_LSQ;
-                    }
-                } else {
-                    sm.I(PI_MODE, p) = MODE_IDLE;
-                }
+                if (nidx >= 0) lane_start<WARM, NC>(prm, sm, c, p, a, nidx, N, batch);
+                else sm.I(PI_MODE, p) = MODE_IDLE;
             }
             fin = false;
         }
@@ -247,63 +201,14 @@ __device__ __forceinline__ void control_loop(const SolveArgs &a, const SM &sm, c
         }
         if (lane) {
             const int md = sm.I(PI_MODE, p);
-            int term = 0;
+            int fl = 0, r = 0;
             if (md == MODE_EVAL) {
-                const int fl = sm.I(PI_FLAGS, p);
-                const int r = ctrl_decide_sums(prm, sm, c, p, fl, sums);
+                fl = sm.I(PI_FLAGS, p);
+                r = ctrl_decide_sums(prm, sm, c, p, fl, sums);
                 PROF_MARK(10);
-                if (r == 0) {
-                    sm.I(PI_FLAGS, p) = FL_LS | (fl & FL_RESTO);
-                } else if (r == 3 || r == 4) {
-                    // second-order correction (3) / resume after failed corrections (4): the same Newton system again
-                    // (PS_DW kept), no step applied
-                    sm.I(PI_MODE, p) = MODE_NEWTON; sm.I(PI_FLAGS, p) = (r == 3) ? FL_SOC : FL_RESUME;
-                } else if (r == 5) {
-                    // the line search failed: feasibility restoration from the iterate (nothing applied)
-                    sm.I(PI_MODE, p) = MODE_NEWTON; sm.I(PI_FLAGS, p) = FL_RESTO; sm.P(PS_DW, p) = 0.0;
-                } else if (r == 6) {
-                    // restoration step taken (primal only), the next restoration system from the new point
-                    sm.P(PS_AP_ALPHA, p) = sm.P(PS_ALPHA, p); sm.P(PS_AP_AZ, p) = NMPC_AZ_RESTO; sm.P(PS_AP_MU, p) = sm.P(PS_MU_STEP, p);
-                    sm.I(PI_MODE, p) = MODE_NEWTON; sm.I(PI_FLAGS, p) = FL_APPLY | FL_RESTO; sm.P(PS_DW, p) = 0.0;
-                } else {
-                    int nf = 0;
-                    // the evaluated point becomes the iterate: P3a applies the step (a plain evaluation is
-                    // a step of length 0 -- it still adopts the sin/cos computed at the evaluated point)
-                    nf = FL_APPLY;
-                    if ((fl & (FL_LS | FL_RESTO)) == (FL_LS | FL_RESTO)) {
-                        // restoration ends here (or the problem does): primal step, multipliers kept, z reset
-                        sm.P(PS_AP_ALPHA, p) = sm.P(PS_ALPHA, p); sm.P(PS_AP_AZ, p) = NMPC_AZ_RESTO_END;
-                    } else if (fl & FL_LS) {
-                        sm.P(PS_AP_ALPHA, p) = sm.P(PS_ALPHA, p); sm.P(PS_AP_AZ, p) = sm.P(PS_ALPHA_Z, p);
-                        ctrl_apply(sm, p);
-                    } else {
-                        sm.P(PS_AP_ALPHA, p) = 0.0; sm.P(PS_AP_AZ, p) = 0.0;
-                    }
-                    sm.P(PS_AP_MU, p) = sm.P(PS_MU_STEP, p);
-                    if (r == 1) { sm.I(PI_MODE, p) = MODE_NEWTON; sm.P(PS_DW, p) = 0.0; sm.I(PI_FLAGS, p) = nf; }
-                    else { term = 1; sm.I(PI_FLAGS, p) = nf | FL_FLUSH; }
-                }
-            } else if (md == MODE_FAIL) {
-                term = 1; sm.I(PI_FLAGS, p) = FL_FLUSH;
             }
-            // watchdog: retries and backtracks are bounded, this only guards against the unforeseen
-            if (!term && md != MODE_IDLE && ++c.age > 8 * prm.max_iter + 64) {
-                if (c.status == 0) c.status = 2;
-                term = 1; sm.I(PI_FLAGS, p) = FL_FLUSH;
-            }
-            if (term) {
-                const size_t i = (size_t)sm.I(PI_PROB, p);
-                if (a.obj) a.obj[i] = c.obj;
-                if (a.status) a.status[i] = c.status;
-                if (a.iters) a.iters[i] = c.iter;
-                if (a.kkt) a.kkt[i] = c.E0;
-                sm.P(PS_AP_SF, p) = sm.P(PS_SF, p);
-                if (a.warm_out) {
-                    const size_t offl = (size_t)(8 * N - 2);
-                    for (int cc = 0; cc < 6; cc++)
-                        a.warm_out[(offl + (size_t)cc * N) * batch + i] = sm.P(PS_L0X + cc, p) / sm.P(PS_SF, p);
-                }
-                sm.I(PI_MODE, p) = MODE_IDLE;
+            if (ctrl_transition(prm, sm, c, p, md, fl, r)) {
+                ctrl_finish(prm, sm, c, p, a, N, batch);
                 fin = true;
             }
         }
@@ -363,21 +268,16 @@ __global__ void __launch_bounds__(NMPC_MAX_THREADS(SPT, CPB), 1) nmpc_solve_kern
                 const int fl = sm.I(PI_FLAGS, p);
                 const int idx = sm.I(PI_NEXT, p);
                 if (idx >= 0) {
-                    double s6[6], c4[4];
-                    for (int i = 0; i < 6; i++) s6[i] = sm.P(PS_NX0 + i, p);
-                    for (int i = 0; i < 4; i++) { c4[i] = sm.P(PS_NX6 + i, p); cf[i] = c4[i]; }
-                    if (NC > 4) {
-#pragma unroll
-                        for (int i = 4; i < NC; i++) cf[i] = sm.P(PS_NXC4 + (i - 4), p);
-                    }
+                    double s6[6];
+                    stage_inputs<NC>(sm, p, s6, cf);
                     if (WARM && (fl & FL_WARM)) {
 #pragma unroll
                         for (int j = 0; j < SPT; j++)
-                            if (k0 + j < N) stage_init_warm<RATE>(prm, sm, r[j], k0 + j, p, s6, c4, a.warm_in, (size_t)batch, (size_t)idx);
+                            if (k0 + j < N) stage_init_warm<RATE>(prm, sm, r[j], k0 + j, p, s6, cf, a.warm_in, (size_t)batch, (size_t)idx);
                     } else {
 #pragma unroll
                         for (int j = 0; j < SPT; j++)
-                            if (k0 + j < N) stage_init<RATE>(prm, sm, r[j], k0 + j, p, s6, c4);
+                            if (k0 + j < N) stage_init<RATE>(prm, sm, r[j], k0 + j, p, s6, cf);
                     }
                 } else if ((fl & (FL_SOC | FL_APPLY)) == FL_SOC && sm.I(PI_MODE, p) == MODE_NEWTON) {
                     // second-order correction: the next right-hand side from the rejected trial point, before the
@@ -464,42 +364,9 @@ __global__ void __launch_bounds__(NMPC_MAX_THREADS(SPT, CPB), 1) nmpc_solve_kern
                         if (k0 + j < N) stage_apply<RATE>(prm, sm, r[j], k0 + j, p);
                 }
                 if (fl & FL_FLUSH) {
-                    // the last iterate whatever the status (mpc_planner.cpp:378-401)
-                    const size_t i = (size_t)sm.I(PI_PROB, p);
 #pragma unroll
-                    for (int j = 0; j < SPT; j++) {
-                        const int k = k0 + j;
-                        if (k >= N) continue;
-                        a.pred[((size_t)0 * N + k) * batch + i] = sm.at(k, S_X, p);
-                        a.pred[((size_t)1 * N + k) * batch + i] = sm.at(k, S_Y, p);
-                        a.pred[((size_t)2 * N + k) * batch + i] = sm.at(k, S_T, p);
-                        if (a.status && stage_bound_hit(prm, sm, k, p)) {
-                            // (the control thread wrote the status before barrier B1b; every stage that hits writes the same value)
-                            const int st = a.status[i];
-                            if (st == 1 || st == 4) a.status[i] = NMPC_STATUS_BOUND_ACTIVE;
-                        }
-                        if (k == 0) { a.u0[i] = r[j].uw; a.u0[(size_t)batch + i] = r[j].ua; }
-                        if (a.warm_out) {
-                            // primal in the reference's variable layout (mpc_planner.cpp:232-239), then equality
-                            // multipliers (row layout of :153-158, unscaled), then zL, zU of w and a.
-                            double *wo = a.warm_out;
-                            const double isf = 1.0 / sm.P(PS_AP_SF, p);
-                            for (int cc = 0; cc < 6; cc++) wo[((size_t)cc * N + k) * batch + i] = sm.at(k, S_X + cc, p);
-                            const size_t offl = (size_t)(8 * N - 2);
-                            if (k < N - 1) {
-                                wo[((size_t)6 * N + k) * batch + i] = r[j].uw;
-                                wo[((size_t)7 * N - 1 + k) * batch + i] = r[j].ua;
-                                for (int cc = 0; cc < 6; cc++)
-                                    wo[(offl + (size_t)cc * N + k + 1) * batch + i] = sm.at(k, L_X + cc, p) * isf;
-                                const size_t offz = offl + (size_t)6 * N;
-                                const int nu = N - 1;
-                                wo[(offz + k) * batch + i] = r[j].zlw * isf;
-                                wo[(offz + nu + k) * batch + i] = r[j].zla * isf;
-                                wo[(offz + 2 * nu + k) * batch + i] = r[j].zuw * isf;
-                                wo[(offz + 3 * nu + k) * batch + i] = r[j].zua * isf;
-                            }
-                        }
-                    }
+                    for (int j = 0; j < SPT; j++)
+                        if (k0 + j < N) stage_flush(prm, sm, r[j], k0 + j, p, a, N, batch);
                 }
             }
         }

@@ -97,37 +97,7 @@ __global__ void __launch_bounds__(384, 1) nmpc_solve_kernel_dual(const SolveArgs
                 if (mine) {
                     const int fl = sm.I(PI_FLAGS, p);
                     if (fl & FL_APPLY) stage_apply<RATE>(prm, sm, r, k, p);
-                    if (fl & FL_FLUSH) {
-                        // the last iterate whatever the status (mpc_planner.cpp:378-401)
-                        const size_t i = (size_t)sm.I(PI_PROB, p);
-                        a.pred[((size_t)0 * N + k) * batch + i] = sm.at(k, S_X, p);
-                        a.pred[((size_t)1 * N + k) * batch + i] = sm.at(k, S_Y, p);
-                        a.pred[((size_t)2 * N + k) * batch + i] = sm.at(k, S_T, p);
-                        if (a.status && stage_bound_hit(prm, sm, k, p)) {
-                            const int st = a.status[i];
-                            if (st == 1 || st == 4) a.status[i] = NMPC_STATUS_BOUND_ACTIVE;
-                        }
-                        if (k == 0) { a.u0[i] = r.uw; a.u0[(size_t)batch + i] = r.ua; }
-                        if (a.warm_out) {
-                            // record layout: see nmpc_kernel.cuh
-                            double *wo = a.warm_out;
-                            const double isf = 1.0 / sm.P(PS_AP_SF, p);
-                            for (int cc = 0; cc < 6; cc++) wo[((size_t)cc * N + k) * batch + i] = sm.at(k, S_X + cc, p);
-                            const size_t offl = (size_t)(8 * N - 2);
-                            if (k < N - 1) {
-                                wo[((size_t)6 * N + k) * batch + i] = r.uw;
-                                wo[((size_t)7 * N - 1 + k) * batch + i] = r.ua;
-                                for (int cc = 0; cc < 6; cc++)
-                                    wo[(offl + (size_t)cc * N + k + 1) * batch + i] = sm.at(k, L_X + cc, p) * isf;
-                                const size_t offz = offl + (size_t)6 * N;
-                                const int nu = N - 1;
-                                wo[(offz + k) * batch + i] = r.zlw * isf;
-                                wo[(offz + nu + k) * batch + i] = r.zla * isf;
-                                wo[(offz + 2 * nu + k) * batch + i] = r.zuw * isf;
-                                wo[(offz + 3 * nu + k) * batch + i] = r.zua * isf;
-                            }
-                        }
-                    }
+                    if (fl & FL_FLUSH) stage_flush(prm, sm, r, k, p, a, N, batch);
                 }
             }
             asm volatile("" ::: "memory");
@@ -140,15 +110,10 @@ __global__ void __launch_bounds__(384, 1) nmpc_solve_kernel_dual(const SolveArgs
                     const int fl = sm.I(PI_FLAGS, p);
                     const int idx = sm.I(PI_NEXT, p);
                     if (idx >= 0) {
-                        double s6[6], c4[4];
-                        for (int i = 0; i < 6; i++) s6[i] = sm.P(PS_NX0 + i, p);
-                        for (int i = 0; i < 4; i++) { c4[i] = sm.P(PS_NX6 + i, p); cf[i] = c4[i]; }
-                        if (NC > 4) {
-#pragma unroll
-                            for (int i = 4; i < NC; i++) cf[i] = sm.P(PS_NXC4 + (i - 4), p);
-                        }
-                        if (WARM && (fl & FL_WARM)) stage_init_warm<RATE>(prm, sm, r, k, p, s6, c4, a.warm_in, (size_t)batch, (size_t)idx);
-                        else stage_init<RATE>(prm, sm, r, k, p, s6, c4);
+                        double s6[6];
+                        stage_inputs<NC>(sm, p, s6, cf);
+                        if (WARM && (fl & FL_WARM)) stage_init_warm<RATE>(prm, sm, r, k, p, s6, cf, a.warm_in, (size_t)batch, (size_t)idx);
+                        else stage_init<RATE>(prm, sm, r, k, p, s6, cf);
                     } else if ((fl & (FL_SOC | FL_APPLY)) == FL_SOC && sm.I(PI_MODE, p) == MODE_NEWTON) {
                         stage_soc_rhs<NC>(prm, sm, r, k, p, cf);
                     }

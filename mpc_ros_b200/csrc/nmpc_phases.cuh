@@ -122,6 +122,28 @@ struct Params {
                           // when the finished problem is written out (stage_bound_hit)
 };
 
+// A batch to solve: inputs, outputs (SoA over the batch) and the work queue.
+struct SolveArgs {
+    Params prm;
+    int PB;
+    int batch;
+    int ncoef;              // rows of coeffs: 4 (cubic) .. NMPC_MAX_COEFFS
+    const double *state;    // 6 x batch
+    const double *coeffs;   // ncoef x batch
+    const double *ref_vel;  // batch or NULL
+    double *u0;             // 2 x batch
+    double *pred;           // 3N x batch
+    double *obj;            // batch or NULL
+    int *status;            // batch or NULL
+    int *iters;             // batch or NULL
+    double *kkt;            // batch or NULL
+    double *warm_out;       // warm_size x batch or NULL
+    const double *warm_in;  // warm_size x batch or NULL (cold start)
+    int *queue;             // work-queue head (zeroed by the host before the launch)
+    const int *order;       // queue position -> problem index (hard-first order) or NULL (identity)
+    long long *prof;        // NMPC_PROFILE builds only: per-phase cycle counters of CTA 0
+};
+
 #define NMPC_MAX_FILTER 8
 // per-problem status outside the solve_result::status_type values: see Params::bound_chk (= MPC_B200_STATUS_BOUND_ACTIVE)
 #define NMPC_STATUS_BOUND_ACTIVE 64
@@ -361,6 +383,15 @@ MPC_HD void stage_init(const Params &prm, const SM &sm, StageRegs &r, int k, int
 // zL_w, zL_a, zU_w, zU_a.  Controls and multipliers are taken from the record (controls pushed into the
 // interior of their bounds); the states are NOT taken from it: the control thread rolls the model out
 // from the given state (ctrl_rollout), so the start point satisfies the dynamics exactly.
+// Rows of the blocks: state c of stage k at c*N + k; controls of stage k < N-1 at warm_uw + k, warm_ua + k; lambda_k,
+// component c, at warm_lam + c*N + k (lambda_0: the initial-condition rows); zL_w, zL_a, zU_w, zU_a of stage k < N-1 at
+// warm_z + j*(N-1) + k, j = 0..3.
+MPC_HD size_t warm_uw(int N) { return (size_t)6 * N; }
+MPC_HD size_t warm_ua(int N) { return (size_t)7 * N - 1; }
+MPC_HD size_t warm_lam(int N) { return (size_t)(8 * N - 2); }
+MPC_HD size_t warm_z(int N) { return warm_lam(N) + (size_t)6 * N; }
+MPC_HD size_t warm_size(int N) { return warm_z(N) + (size_t)4 * (N - 1); }
+
 template <bool RATE = false, class SM>
 MPC_HD void stage_init_warm(const Params &prm, const SM &sm, StageRegs &r, int k, int p,
                             const double *state6, const double *coef4, const double *warm, size_t stride, size_t idx)
@@ -370,13 +401,13 @@ MPC_HD void stage_init_warm(const Params &prm, const SM &sm, StageRegs &r, int k
     if (k < N - 1) {
         const double sf = sm.P(PS_SF, p), mu = prm.warm_mu;
         const double Uw = relaxed(prm.max_angvel), Ua = relaxed(prm.max_throttle);
-        double uw = warm[((size_t)6 * N + k) * stride + idx], ua = warm[((size_t)7 * N - 1 + k) * stride + idx];
+        double uw = warm[(warm_uw(N) + k) * stride + idx], ua = warm[(warm_ua(N) + k) * stride + idx];
         const double pw = 1e-3 * Uw, pa = 1e-3 * Ua;       // warm_start_bound_push
         uw = fmax2(fmin2(uw, Uw - pw), -Uw + pw); ua = fmax2(fmin2(ua, Ua - pa), -Ua + pa);
         r.uw = uw; r.ua = ua;
         sm.at(k, W_10, p) = uw; sm.at(k, W_11, p) = ua;    // for the roll-out
         if (RATE) { sm.at(k, U_W, p) = uw; sm.at(k, U_A, p) = ua; }
-        const size_t offl = (size_t)(8 * N - 2), offz = offl + (size_t)6 * N;
+        const size_t offl = warm_lam(N), offz = warm_z(N);
         for (int c = 0; c < 6; c++) sm.at(k, L_X + c, p) = sf * warm[(offl + (size_t)c * N + k + 1) * stride + idx];
         const int nu = N - 1;
         // multipliers of the control bounds: at least on the central path of the starting mu
@@ -1615,6 +1646,152 @@ MPC_HD void ctrl_apply(const SM &sm, int p)
     for (int i = 0; i < 6; i++) {
         const double l = sm.P(PS_L0X + i, p);
         sm.P(PS_L0X + i, p) = l + alpha * (sm.P(PS_N0X + i, p) - l);
+    }
+}
+
+// ---------------------------------------------------------------- lane transitions, start and write-out of a problem
+// The helpers that read or write the batch's arrays take N = prm.N and batch = a.batch as the caller holds them: the kernels
+// load both once, and reading them from the arguments again here would keep the compiler from hoisting the index arithmetic.
+//
+// Refill, control side: problem nidx (after the a.order mapping) takes over lane p.  Its inputs are staged in PS_NX* for
+// the stage threads (stage_inputs, P3a); the first cycle rolls a warm start out, or solves the least-squares multiplier
+// system of a cold start.
+template <bool WARM, int NC, class SM>
+MPC_HD void lane_start(const Params &prm, const SM &sm, Ctrl &c, int p, const SolveArgs &a, int nidx, const int N, const int batch)
+{
+    for (int i = 0; i < 6; i++) sm.P(PS_NX0 + i, p) = a.state[(size_t)i * batch + nidx];
+    for (int i = 0; i < 4; i++) sm.P(PS_NX6 + i, p) = a.coeffs[(size_t)i * batch + nidx];
+    if (NC > 4)
+        for (int i = 4; i < NC; i++)
+            sm.P(PS_NXC4 + (i - 4), p) = i < a.ncoef ? a.coeffs[(size_t)i * batch + nidx] : 0.0;
+    sm.P(PS_NX10, p) = a.ref_vel ? a.ref_vel[nidx] : prm.ref_vel;
+    double s6[6];
+    for (int i = 0; i < 6; i++) s6[i] = sm.P(PS_NX0 + i, p);
+    ctrl_init(prm, sm, c, p, s6, sm.P(PS_NX10, p));
+    if (WARM) {
+        sm.P(PS_MU, p) = prm.warm_mu; sm.P(PS_MU_STEP, p) = prm.warm_mu;
+        sm.P(PS_TAU, p) = fmax2(NMPC_TAU_MIN, 1.0 - prm.warm_mu);
+        const size_t offl = warm_lam(N);
+        for (int i = 0; i < 6; i++)
+            sm.P(PS_L0X + i, p) = sm.P(PS_SF, p) * a.warm_in[(offl + (size_t)i * N) * batch + nidx];
+        sm.I(PI_MODE, p) = MODE_ROLLOUT;
+        sm.I(PI_FLAGS, p) |= FL_WARM;
+    } else {
+        sm.I(PI_MODE, p) = MODE_NEWTON;
+        sm.I(PI_FLAGS, p) |= FL_LSQ;
+    }
+}
+
+// P3a, stage side: the state and path polynomial lane_start staged (cf[0..3] is the cubic part).
+template <int NC, class SM>
+MPC_HD void stage_inputs(const SM &sm, int p, double *s6, double *cf)
+{
+    for (int i = 0; i < 6; i++) s6[i] = sm.P(PS_NX0 + i, p);
+    for (int i = 0; i < 4; i++) cf[i] = sm.P(PS_NX6 + i, p);
+#pragma unroll
+    for (int i = 4; i < NC; i++) cf[i] = sm.P(PS_NXC4 + (i - 4), p);
+}
+
+// P2, after the decision r = ctrl_decide (md == MODE_EVAL; fl: the flags it decided with): the lane's next mode and flags,
+// and in PS_AP_* the step P3a0 applies.  Returns 1 when the lane's problem terminates (then ctrl_finish).
+template <class SM>
+MPC_HD int ctrl_transition(const Params &prm, const SM &sm, Ctrl &c, int p, int md, int fl, int r)
+{
+    int term = 0;
+    if (md == MODE_EVAL) {
+        if (r == 0) {
+            sm.I(PI_FLAGS, p) = FL_LS | (fl & FL_RESTO);
+        } else if (r == 3 || r == 4) {
+            // second-order correction (3) / resume after failed corrections (4): the same Newton system again
+            // (PS_DW kept), no step applied
+            sm.I(PI_MODE, p) = MODE_NEWTON; sm.I(PI_FLAGS, p) = (r == 3) ? FL_SOC : FL_RESUME;
+        } else if (r == 5) {
+            // the line search failed: feasibility restoration from the iterate (nothing applied)
+            sm.I(PI_MODE, p) = MODE_NEWTON; sm.I(PI_FLAGS, p) = FL_RESTO; sm.P(PS_DW, p) = 0.0;
+        } else if (r == 6) {
+            // restoration step taken (primal only), the next restoration system from the new point
+            sm.P(PS_AP_ALPHA, p) = sm.P(PS_ALPHA, p); sm.P(PS_AP_AZ, p) = NMPC_AZ_RESTO; sm.P(PS_AP_MU, p) = sm.P(PS_MU_STEP, p);
+            sm.I(PI_MODE, p) = MODE_NEWTON; sm.I(PI_FLAGS, p) = FL_APPLY | FL_RESTO; sm.P(PS_DW, p) = 0.0;
+        } else {
+            // the evaluated point becomes the iterate: P3a applies the step (a plain evaluation is
+            // a step of length 0 -- it still adopts the sin/cos computed at the evaluated point)
+            const int nf = FL_APPLY;
+            if ((fl & (FL_LS | FL_RESTO)) == (FL_LS | FL_RESTO)) {
+                // restoration ends here (or the problem does): primal step, multipliers kept, z reset
+                sm.P(PS_AP_ALPHA, p) = sm.P(PS_ALPHA, p); sm.P(PS_AP_AZ, p) = NMPC_AZ_RESTO_END;
+            } else if (fl & FL_LS) {
+                sm.P(PS_AP_ALPHA, p) = sm.P(PS_ALPHA, p); sm.P(PS_AP_AZ, p) = sm.P(PS_ALPHA_Z, p);
+                ctrl_apply(sm, p);
+            } else {
+                sm.P(PS_AP_ALPHA, p) = 0.0; sm.P(PS_AP_AZ, p) = 0.0;
+            }
+            sm.P(PS_AP_MU, p) = sm.P(PS_MU_STEP, p);
+            if (r == 1) { sm.I(PI_MODE, p) = MODE_NEWTON; sm.P(PS_DW, p) = 0.0; sm.I(PI_FLAGS, p) = nf; }
+            else { term = 1; sm.I(PI_FLAGS, p) = nf | FL_FLUSH; }
+        }
+    } else if (md == MODE_FAIL) {
+        term = 1; sm.I(PI_FLAGS, p) = FL_FLUSH;
+    }
+    // watchdog: retries and backtracks are bounded, this only guards against the unforeseen
+    if (!term && md != MODE_IDLE && ++c.age > 8 * prm.max_iter + 64) {
+        if (c.status == 0) c.status = 2;
+        term = 1; sm.I(PI_FLAGS, p) = FL_FLUSH;
+    }
+    return term;
+}
+
+// P2, the lane's problem has terminated: its scalar results and lambda_0 (unscaled) are written out, and the lane idles.
+// The stage threads flush the last iterate in the next P3a0 (stage_flush), with the scaling kept in PS_AP_SF.
+template <class SM>
+MPC_HD void ctrl_finish(const Params &prm, const SM &sm, const Ctrl &c, int p, const SolveArgs &a, const int N, const int batch)
+{
+    const size_t i = (size_t)sm.I(PI_PROB, p);
+    if (a.obj) a.obj[i] = c.obj;
+    if (a.status) a.status[i] = c.status;
+    if (a.iters) a.iters[i] = c.iter;
+    if (a.kkt) a.kkt[i] = c.E0;
+    sm.P(PS_AP_SF, p) = sm.P(PS_SF, p);
+    if (a.warm_out) {
+        const size_t offl = warm_lam(N);
+        for (int cc = 0; cc < 6; cc++)
+            a.warm_out[(offl + (size_t)cc * N) * batch + i] = sm.P(PS_L0X + cc, p) / sm.P(PS_SF, p);
+    }
+    sm.I(PI_MODE, p) = MODE_IDLE;
+}
+
+// P3a0, stage k of a finished problem: the last iterate whatever the status (mpc_planner.cpp:378-401).  Runs after
+// ctrl_finish has written the status.
+template <class SM>
+MPC_HD void stage_flush(const Params &prm, const SM &sm, const StageRegs &r, int k, int p, const SolveArgs &a, const int N, const int batch)
+{
+    const size_t i = (size_t)sm.I(PI_PROB, p);
+    a.pred[((size_t)0 * N + k) * batch + i] = sm.at(k, S_X, p);
+    a.pred[((size_t)1 * N + k) * batch + i] = sm.at(k, S_Y, p);
+    a.pred[((size_t)2 * N + k) * batch + i] = sm.at(k, S_T, p);
+    if (a.status && stage_bound_hit(prm, sm, k, p)) {
+        // (every stage that hits writes the same value)
+        const int st = a.status[i];
+        if (st == 1 || st == 4) a.status[i] = NMPC_STATUS_BOUND_ACTIVE;
+    }
+    if (k == 0) { a.u0[i] = r.uw; a.u0[(size_t)batch + i] = r.ua; }
+    if (a.warm_out) {
+        // the warm-start record (layout: stage_init_warm), multipliers unscaled
+        double *wo = a.warm_out;
+        const double isf = 1.0 / sm.P(PS_AP_SF, p);
+        for (int cc = 0; cc < 6; cc++) wo[((size_t)cc * N + k) * batch + i] = sm.at(k, S_X + cc, p);
+        const size_t offl = warm_lam(N);
+        if (k < N - 1) {
+            wo[(warm_uw(N) + k) * batch + i] = r.uw;
+            wo[(warm_ua(N) + k) * batch + i] = r.ua;
+            for (int cc = 0; cc < 6; cc++)
+                wo[(offl + (size_t)cc * N + k + 1) * batch + i] = sm.at(k, L_X + cc, p) * isf;
+            const size_t offz = warm_z(N);
+            const int nu = N - 1;
+            wo[(offz + k) * batch + i] = r.zlw * isf;
+            wo[(offz + nu + k) * batch + i] = r.zla * isf;
+            wo[(offz + 2 * nu + k) * batch + i] = r.zuw * isf;
+            wo[(offz + 3 * nu + k) * batch + i] = r.zua * isf;
+        }
     }
 }
 

@@ -1,10 +1,11 @@
 // tests/emu/nmpc_emu.cpp -- TEST INFRASTRUCTURE, NOT PRODUCT CODE.
 //
 // Runs the solver's phase functions (mpc_ros_b200/csrc/nmpc_phases.cuh, the code the CUDA
-// kernel executes) sequentially on the host, one emulated CTA of PB lanes at a time, with the
-// kernel's cycle / barrier structure (nmpc_kernel.cuh) turned into plain loops -- including the
-// per-lane state machine.  (The kernel's work queue is not emulated: lanes get their problems
-// statically; results do not depend on the lane, which the tests check.)  It exists so that the
+// kernel executes: the arithmetic, the per-lane state machine, the start of a problem in a lane and
+// the write-out of its results) sequentially on the host, one emulated CTA of PB lanes at a time, with
+// the kernel's cycle / barrier structure (nmpc_kernel.cuh) turned into plain loops.  (The kernel's
+// work queue is not emulated: lanes get their problems statically; results do not depend on the
+// lane, which the tests check.)  It exists so that the
 // solver LOGIC can be checked against the oracle in the CPU-only test tier (this container has no
 // GPU).  It is built only by tests/ into tests/emu/libnmpc_emu.so, is never linked into
 // libmpc_b200.so, and nothing in the product path can reach it.
@@ -19,13 +20,16 @@ static std::vector<int> g_ages, g_kinds;   // g_kinds: 4 per problem: backtracks
 static std::vector<int> g_kind_lane;
 static std::vector<int> g_ages_unused;      // global cycles each problem of the last run took (tail studies)
 
-template <bool RATE, int NC = 4>
-static int emu_run(int N, const double *prm14, double tol, int max_iter, int PB, int batch, int ncoef,
-                   const double *state, const double *coeffs, const double *ref_vel,
-                   double *u0, double *pred, double *obj, int *status, int *iters, double *kkt,
-                   double *lam_out, int *n_reg)
+static const int SPT = 2;   // same grouping of partial sums as the kernel's stage threads
+
+// The kernel's arguments for one batch.  prm14: dt, ref_cte, ref_etheta, ref_vel, w_cte, w_etheta, w_vel, w_angvel,
+// w_accel, max_angvel, max_throttle, w_angvel_d, w_accel_d, bound_value (0 = the 1e3 default).
+static SolveArgs emu_args(int N, const double *prm14, double tol, int max_iter, int PB, int batch, int ncoef,
+                          const double *state, const double *coeffs, const double *ref_vel,
+                          double *u0, double *pred, double *obj, int *status, int *iters, double *kkt, double *warm_out)
 {
-    Params prm;
+    SolveArgs a = {};
+    Params &prm = a.prm;
     prm.N = N;
     prm.dt = prm14[0]; prm.ref_cte = prm14[1]; prm.ref_etheta = prm14[2]; prm.ref_vel = prm14[3];
     prm.w_cte = prm14[4]; prm.w_etheta = prm14[5]; prm.w_vel = prm14[6]; prm.w_angvel = prm14[7];
@@ -33,11 +37,21 @@ static int emu_run(int N, const double *prm14, double tol, int max_iter, int PB,
     prm.tol = tol; prm.max_iter = max_iter;
     prm.warm_mu = 1e-3;
     prm.w_angvel_d = prm14[11]; prm.w_accel_d = prm14[12];
-    const int SPT = 2;   // same grouping of partial sums as the kernel's stage threads
     prm.grp = SPT;
     prm.idt = 1.0 / prm.dt;
     prm.i_mnb = 1.0 / (double)(6 * N + 4 * (N - 1)); prm.i_nb = 1.0 / (double)(4 * (N - 1));
-    prm.bound_chk = (prm14[13] > 0.0 ? prm14[13] : 1e3) * (1.0 - 1e-3);   // prm14[13]: bound_value (0 = the 1e3 default)
+    prm.bound_chk = (prm14[13] > 0.0 ? prm14[13] : 1e3) * (1.0 - 1e-3);
+    a.PB = PB; a.batch = batch; a.ncoef = ncoef;
+    a.state = state; a.coeffs = coeffs; a.ref_vel = ref_vel;
+    a.u0 = u0; a.pred = pred; a.obj = obj; a.status = status; a.iters = iters; a.kkt = kkt; a.warm_out = warm_out;
+    return a;
+}
+
+template <bool RATE, int NC = 4>
+static int emu_run(const SolveArgs &a, int *n_reg)
+{
+    const Params &prm = a.prm;
+    const int N = prm.N, PB = a.PB, batch = a.batch;
     const int NG = (N + SPT - 1) / SPT;
     g_ages.assign((size_t)batch, 0); g_kinds.assign((size_t)4 * batch, 0); g_kind_lane.assign((size_t)4 * PB, 0);
 
@@ -56,12 +70,8 @@ static int emu_run(int N, const double *prm14, double tol, int max_iter, int PB,
         for (int p = 0; p < PB; p++) { sm.I(PI_MODE, p) = MODE_IDLE; sm.I(PI_FLAGS, p) = 0; sm.I(PI_PROB, p) = -1; sm.I(PI_NEXT, p) = -1; }
         // ---- "refill": every lane starts its problem
         for (int p = 0; p < np; p++) {
-            double s6[6];
-            for (int c = 0; c < 6; c++) s6[c] = state[(size_t)c * batch + base + p];
-            const double rv = ref_vel ? ref_vel[base + p] : prm.ref_vel;
-            ctrl_init(prm, sm, ctrl[p], p, s6, rv);
             sm.I(PI_NEXT, p) = base + p;
-            sm.I(PI_MODE, p) = MODE_NEWTON; sm.I(PI_FLAGS, p) = FL_LSQ;
+            lane_start<false, NC>(prm, sm, ctrl[p], p, a, base + p, N, batch);
             nreg[p] = 0; for (int q = 0; q < 4; q++) g_kind_lane[4 * p + q] = 0;
         }
         for (;;) {
@@ -73,33 +83,11 @@ static int emu_run(int N, const double *prm14, double tol, int max_iter, int PB,
             for (int p = 0; p < np; p++) {
                 const int fl = sm.I(PI_FLAGS, p);
                 if (fl & FL_APPLY) for (int k = 0; k < N; k++) stage_apply<RATE>(prm, sm, REG(k, p), k, p);
-                if (fl & FL_FLUSH) {
-                    const size_t i = (size_t)sm.I(PI_PROB, p);
-                    if (status)
-                        for (int k = 0; k < N; k++)
-                            if (stage_bound_hit(prm, sm, k, p) && (status[i] == 1 || status[i] == 4)) status[i] = NMPC_STATUS_BOUND_ACTIVE;
-                    u0[i] = REG(0, p).uw; u0[(size_t)batch + i] = REG(0, p).ua;
-                    for (int k = 0; k < N; k++) {
-                        pred[((size_t)0 * N + k) * batch + i] = sm.at(k, S_X, p);
-                        pred[((size_t)1 * N + k) * batch + i] = sm.at(k, S_Y, p);
-                        pred[((size_t)2 * N + k) * batch + i] = sm.at(k, S_T, p);
-                    }
-                    if (lam_out) {
-                        const double sf = sm.P(PS_AP_SF, p);
-                        for (int c = 0; c < 6; c++)
-                            for (int k = 0; k < N - 1; k++)
-                                lam_out[((size_t)c * N + k + 1) * batch + i] = sm.at(k, L_X + c, p) / sf;
-                    }
-                }
-                const int idx = sm.I(PI_NEXT, p);
-                if (idx >= 0) {
-                    double s6[6], c4[4];
-                    for (int c = 0; c < 6; c++) s6[c] = state[(size_t)c * batch + idx];
-                    for (int c = 0; c < 4; c++) c4[c] = coeffs[(size_t)c * batch + idx];
-                    for (int c = 0; c < NC; c++) cfs[(size_t)NC * p + c] = c < ncoef ? coeffs[(size_t)c * batch + idx] : 0.0;
-                    for (int c = 0; c < 4; c++) sm.P(PS_NX6 + c, p) = c4[c];        // (the kernel's refill stages them here)
-                    for (int c = 4; c < NC; c++) sm.P(PS_NXC4 + (c - 4), p) = c < ncoef ? coeffs[(size_t)c * batch + idx] : 0.0;
-                    for (int k = 0; k < N; k++) stage_init<RATE>(prm, sm, REG(k, p), k, p, s6, c4);
+                if (fl & FL_FLUSH) for (int k = 0; k < N; k++) stage_flush(prm, sm, REG(k, p), k, p, a, N, batch);
+                if (sm.I(PI_NEXT, p) >= 0) {
+                    double s6[6];
+                    stage_inputs<NC>(sm, p, s6, &cfs[(size_t)NC * p]);
+                    for (int k = 0; k < N; k++) stage_init<RATE>(prm, sm, REG(k, p), k, p, s6, &cfs[(size_t)NC * p]);
                 }
             }
             // second-order correction: next right-hand side from the rejected trial point, before any stage's coefficients
@@ -180,58 +168,19 @@ static int emu_run(int N, const double *prm14, double tol, int max_iter, int PB,
             for (int p = 0; p < np; p++) {
                 Ctrl &c = ctrl[p];
                 const int md = sm.I(PI_MODE, p);
-                int term = 0;
+                int fl = 0, r = 0;
                 if (md == MODE_EVAL) {
-                    const int fl = sm.I(PI_FLAGS, p);
-                    const int r = ctrl_decide(prm, sm, c, p, fl, NG);
+                    fl = sm.I(PI_FLAGS, p);
+                    r = ctrl_decide(prm, sm, c, p, fl, NG);
                     if (r == 0) g_kind_lane[4 * p]++; else if (r == 3) g_kind_lane[4 * p + 1]++; else if (r == 4) g_kind_lane[4 * p + 2]++;
                     if (r == 5 || r == 6) g_kind_lane[4 * p + 1]++;      // (restoration steps are counted with the corrections)
-                    if (r == 0) sm.I(PI_FLAGS, p) = FL_LS | (fl & FL_RESTO);
-                    else if (r == 3) { sm.I(PI_MODE, p) = MODE_NEWTON; sm.I(PI_FLAGS, p) = FL_SOC; }
-                    else if (r == 4) { sm.I(PI_MODE, p) = MODE_NEWTON; sm.I(PI_FLAGS, p) = FL_RESUME; }
-                    else if (r == 5) { sm.I(PI_MODE, p) = MODE_NEWTON; sm.I(PI_FLAGS, p) = FL_RESTO; sm.P(PS_DW, p) = 0.0; }
-                    else if (r == 6) {
-                        sm.P(PS_AP_ALPHA, p) = sm.P(PS_ALPHA, p); sm.P(PS_AP_AZ, p) = NMPC_AZ_RESTO; sm.P(PS_AP_MU, p) = sm.P(PS_MU_STEP, p);
-                        sm.I(PI_MODE, p) = MODE_NEWTON; sm.I(PI_FLAGS, p) = FL_APPLY | FL_RESTO; sm.P(PS_DW, p) = 0.0;
-                    } else {
-                        int nf = 0;
-                        // the evaluated point becomes the iterate: P3a applies the step (a plain evaluation is
-                        // a step of length 0 -- it still adopts the sin/cos computed at the evaluated point)
-                        nf = FL_APPLY;
-                        if ((fl & (FL_LS | FL_RESTO)) == (FL_LS | FL_RESTO)) {
-                            sm.P(PS_AP_ALPHA, p) = sm.P(PS_ALPHA, p); sm.P(PS_AP_AZ, p) = NMPC_AZ_RESTO_END;
-                        } else if (fl & FL_LS) {
-                            sm.P(PS_AP_ALPHA, p) = sm.P(PS_ALPHA, p); sm.P(PS_AP_AZ, p) = sm.P(PS_ALPHA_Z, p);
-                            ctrl_apply(sm, p);
-                        } else {
-                            sm.P(PS_AP_ALPHA, p) = 0.0; sm.P(PS_AP_AZ, p) = 0.0;
-                        }
-                        sm.P(PS_AP_MU, p) = sm.P(PS_MU_STEP, p);
-                        if (r == 1) { sm.I(PI_MODE, p) = MODE_NEWTON; sm.P(PS_DW, p) = 0.0; sm.I(PI_FLAGS, p) = nf; }
-                        else { term = 1; sm.I(PI_FLAGS, p) = nf | FL_FLUSH; }
-                    }
-                } else if (md == MODE_FAIL) {
-                    term = 1; sm.I(PI_FLAGS, p) = FL_FLUSH;
                 }
-                // watchdog: retries and backtracks are bounded, this only guards against the unforeseen
-                if (!term && md != MODE_IDLE && ++c.age > 8 * prm.max_iter + 64) {
-                    if (c.status == 0) c.status = 2;
-                    term = 1; sm.I(PI_FLAGS, p) = FL_FLUSH;
-                }
-                if (term) {
+                if (ctrl_transition(prm, sm, c, p, md, fl, r)) {
                     const size_t i = (size_t)sm.I(PI_PROB, p);
-                    if (obj) obj[i] = c.obj;
-                    if (status) status[i] = c.status;
-                    if (iters) iters[i] = c.iter;
-                    if (kkt) kkt[i] = c.E0;
                     if (n_reg) n_reg[i] = nreg[p];
                     g_ages[i] = c.age + 1; g_kind_lane[4 * p + 3] = nreg[p];
                     for (int q = 0; q < 4; q++) g_kinds[4 * i + q] = g_kind_lane[4 * p + q];
-                    sm.P(PS_AP_SF, p) = sm.P(PS_SF, p);
-                    if (lam_out)
-                        for (int cc = 0; cc < 6; cc++)
-                            lam_out[((size_t)cc * N) * batch + i] = sm.P(PS_L0X + cc, p) / sm.P(PS_SF, p);
-                    sm.I(PI_MODE, p) = MODE_IDLE;
+                    ctrl_finish(prm, sm, c, p, a, N, batch);
                 }
             }
         }
@@ -249,14 +198,13 @@ extern "C" long long nmpc_emu_lane_cycles(int reset) { const long long v = g_lan
 extern "C" int nmpc_emu_solve(int N, const double *prm14, double tol, int max_iter, int PB, int batch,
                               const double *state, const double *coeffs, const double *ref_vel,
                               double *u0, double *pred, double *obj, int *status, int *iters, double *kkt,
-                              double *lam_out /* 6N x batch, optional */, int *n_reg /* batch, optional */)
+                              double *warm_out /* warm_size x batch, optional */, int *n_reg /* batch, optional */)
 {
+    const SolveArgs a = emu_args(N, prm14, tol, max_iter, PB, batch, 4, state, coeffs, ref_vel, u0, pred, obj, status, iters, kkt,
+                                 warm_out);
     // prm14[11], prm14[12]: w_angvel_d, w_accel_d (rate penalties) select the augmented-Riccati variant
-    if (prm14[11] != 0.0 || prm14[12] != 0.0)
-        return emu_run<true>(N, prm14, tol, max_iter, PB, batch, 4, state, coeffs, ref_vel, u0, pred, obj, status, iters, kkt,
-                             lam_out, n_reg);
-    return emu_run<false>(N, prm14, tol, max_iter, PB, batch, 4, state, coeffs, ref_vel, u0, pred, obj, status, iters, kkt,
-                          lam_out, n_reg);
+    if (prm14[11] != 0.0 || prm14[12] != 0.0) return emu_run<true>(a, n_reg);
+    return emu_run<false>(a, n_reg);
 }
 
 // Path polynomial of order ncoef - 1 in 4 .. NMPC_MAX_COEFFS - 1 (coeffs: ncoef x batch): the instantiation the
@@ -266,9 +214,8 @@ extern "C" int nmpc_emu_solve_poly(int N, const double *prm14, double tol, int m
                                    int *status, int *iters, double *kkt)
 {
     if (ncoef < 4 || ncoef > NMPC_MAX_COEFFS) return -1;
-    if (prm14[11] != 0.0 || prm14[12] != 0.0)
-        return emu_run<true, NMPC_MAX_COEFFS>(N, prm14, tol, max_iter, PB, batch, ncoef, state, coeffs, nullptr, u0, pred, obj,
-                                              status, iters, kkt, nullptr, nullptr);
-    return emu_run<false, NMPC_MAX_COEFFS>(N, prm14, tol, max_iter, PB, batch, ncoef, state, coeffs, nullptr, u0, pred, obj,
-                                           status, iters, kkt, nullptr, nullptr);
+    const SolveArgs a = emu_args(N, prm14, tol, max_iter, PB, batch, ncoef, state, coeffs, nullptr, u0, pred, obj, status, iters,
+                                 kkt, nullptr);
+    if (prm14[11] != 0.0 || prm14[12] != 0.0) return emu_run<true, NMPC_MAX_COEFFS>(a, nullptr);
+    return emu_run<false, NMPC_MAX_COEFFS>(a, nullptr);
 }

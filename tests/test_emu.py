@@ -6,6 +6,7 @@ import os
 
 import numpy as np
 
+from mpc_ros_b200 import capi
 from oracle.oracle_py import YAML_DEFAULT, CFG_DEFAULT
 from tests.problems import mild, generated, restoration_cases
 
@@ -23,14 +24,16 @@ def emu_solve(pm, state, coeffs, PB=4, tol=1e-8, max_iter=200, ref_vel=None):
                     min(pm.get("BOUND", 1e3), 1e300)],
                    dtype=np.float64)
     state = np.ascontiguousarray(state, dtype=np.float64); coeffs = np.ascontiguousarray(coeffs, dtype=np.float64)
-    u0 = np.zeros((2, B)); pred = np.zeros((3 * N, B)); obj = np.zeros(B); kkt = np.zeros(B); lam = np.zeros((6 * N, B))
+    u0 = np.zeros((2, B)); pred = np.zeros((3 * N, B)); obj = np.zeros(B); kkt = np.zeros(B)
+    warm = np.zeros((capi.lib().mpc_b200_warm_size(N), B))     # the kernel's warm-start record
     st = np.zeros(B, dtype=np.int32); it = np.zeros(B, dtype=np.int32); nreg = np.zeros(B, dtype=np.int32)
     rv = None if ref_vel is None else np.ascontiguousarray(ref_vel, dtype=np.float64).ctypes.data_as(dp)
     P = lambda a: a.ctypes.data_as(dp)  # noqa: E731
     _EMU.nmpc_emu_solve(C.c_int(N), P(prm), C.c_double(tol), C.c_int(max_iter), C.c_int(PB), C.c_int(B), P(state),
                         P(coeffs), rv, P(u0), P(pred), P(obj), st.ctypes.data_as(ip), it.ctypes.data_as(ip), P(kkt),
-                        P(lam), nreg.ctypes.data_as(ip))
-    return dict(u0=u0, pred=pred, obj=obj, status=st, iters=it, kkt=kkt, lam=lam, nreg=nreg)
+                        P(warm), nreg.ctypes.data_as(ip))
+    n = 8 * N - 2       # equality multipliers: rows [n, n + 6N) of the record
+    return dict(u0=u0, pred=pred, obj=obj, status=st, iters=it, kkt=kkt, lam=warm[n:n + 6 * N], warm=warm, nreg=nreg)
 
 
 def test_emu_matches_oracle_mild(oracle):
@@ -50,6 +53,27 @@ def test_emu_matches_oracle_mild(oracle):
         assert np.abs(r["u0"][:, i] - o2["u0"]).max() <= 1e-10
         assert np.abs(r["lam"][:, i] - o2["lam"]).max() <= 1e-8 * max(1.0, np.abs(o2["lam"]).max())
         assert np.abs(r["pred"][:, i].reshape(3, -1) - o["pred"]).max() <= 1e-6
+
+
+def test_emu_warm_record_matches_oracle(oracle):
+    """The whole warm-start record the kernel's write-out fills (primal, equality multipliers, control-bound multipliers,
+    all unscaled) against the oracle's solution without the (inactive) state bounds: same iterates, so equal to rounding."""
+    pm = dict(YAML_DEFAULT, BOUND=1e19)
+    N = int(pm["STEPS"]); n = 8 * N - 2; m = 6 * N; nu = N - 1
+    w, a = slice(6 * N, 7 * N - 1), slice(7 * N - 1, n)        # the controls in the reference's variable layout
+    state, coeffs = mild(27, 12)
+    r = emu_solve(pm, state, coeffs, PB=5)
+    assert r["warm"].shape[0] == n + m + 4 * nu
+    close = lambda x, ref: np.abs(x - ref).max() <= 1e-8 * max(1.0, np.abs(ref).max())  # noqa: E731
+    for i in range(12):
+        o = oracle.solve(pm, state[:, i], coeffs[:, i])
+        assert r["status"][i] == 1 and o["status"] == 1
+        rec = r["warm"][:, i]
+        assert close(rec[:n], o["sol"])
+        assert close(rec[n:n + m], o["lam"])
+        zlw, zla, zuw, zua = (rec[n + m + j * nu:n + m + (j + 1) * nu] for j in range(4))
+        assert close(zlw, o["zl"][w]) and close(zla, o["zl"][a])
+        assert close(zuw, o["zu"][w]) and close(zua, o["zu"][a])
 
 
 def test_emu_matches_oracle_generated(oracle):
