@@ -19,6 +19,10 @@
 // for the slowest problem of a batch (iteration counts range from 5 to the cap).
 // The control warp's serial chain bounds the cycle, so what need not be on it runs beside it: the adjoint
 // sweep on the lane's stage thread of group 0 (P6), apply / flush on the stage threads during the refill.
+// What a lane does in each phase (the stages_* / stage_adjoint helpers of the stage threads, the ctrl_* helpers of
+// the control thread, the lane start and the write-out) is in nmpc_phases.cuh, shared with the dual-group kernel
+// and the host emulator (tests/emu).  This file keeps the barriers, the work-queue pop, the vote, the P2 reduction,
+// the warm roll-out and the profiling marks.
 //
 // Replaces, per problem: CppAD::ipopt::solve + Ipopt (mpc_ros/src/mpc_planner.cpp:373-375).
 #pragma once
@@ -117,35 +121,20 @@ __device__ __forceinline__ void control_loop(const SolveArgs &a, const SM &sm, c
         // ---- P3a: stage threads apply / flush / init
         cta_sync<DUAL>(bar_id, bar_count);  // B3
         TRACE_C(2);
-        if (lane) {   // apply / flush / init are done (FL_SOC next to FL_APPLY: the applied step was a correction)
-            const int f0 = sm.I(PI_FLAGS, p);
-            sm.I(PI_FLAGS, p) = f0 & ~(FL_APPLY | FL_FLUSH | FL_WARM | ((f0 & FL_APPLY) ? FL_SOC : 0));
-            if (sm.I(PI_NEXT, p) >= 0) { sm.I(PI_PROB, p) = sm.I(PI_NEXT, p); sm.I(PI_NEXT, p) = -1; }
-        }
+        if (lane) ctrl_handover(sm, p);
         // ---- P3b: stage threads write coefficients
         cta_sync<DUAL>(bar_id, bar_count);  // B4
         TRACE_C(3);
         PROF_MARK(2);
         // ---- P4: Riccati sweeps
         int step_lsq = 0;     // sampled here for P6: the lane's adjoint stage thread rewrites PI_FLAGS there
-        int step_mode = 0;    // FL_SOC / FL_RESUME of the system being solved
+        int step_mode = 0;    // FL_SOC / FL_RESUME / FL_RESTO of the system being solved
         if (lane && sm.I(PI_MODE, p) == MODE_NEWTON) {
-            const int lsq = sys_kind(sm.I(PI_FLAGS, p));      // 0 Newton step, 1 least-squares start, 2 restoration step
-            step_lsq = lsq == 1;
-            step_mode = sm.I(PI_FLAGS, p) & (FL_SOC | FL_RESUME | FL_RESTO);
-            const double dw = sm.P(PS_DW, p);
-            const HessDiag hd = hess_diag(prm, sm.P(PS_SF, p), dw, lsq);
-            const int okb = riccati_backward<RATE>(prm, sm, p, hd);
+            const NewtonSys ns = ctrl_newton_backward<RATE>(prm, sm, p);
             PROF_MARK(3);
-            if (okb || lsq) {
-                riccati_forward<RATE>(prm, sm, p, hd);
-                if (dw > 0.0) c.dw_last = dw;
-                sm.I(PI_MODE, p) = MODE_STEP;
-            } else {
-                const double nd = next_dw(c, dw);
-                if (nd > NMPC_DW_MAX) { c.status = 10; sm.I(PI_MODE, p) = MODE_FAIL; }
-                else sm.P(PS_DW, p) = nd;       // stays MODE_NEWTON: coefficients are rewritten next cycle
-            }
+            ctrl_newton_forward<RATE>(prm, sm, c, p, ns);
+            step_lsq = ns.lsq == 1;
+            step_mode = ns.mode;
         }
         if (WARM && lane && sm.I(PI_MODE, p) == MODE_ROLLOUT) {
             const size_t i = (size_t)sm.I(PI_PROB, p);
@@ -167,14 +156,7 @@ __device__ __forceinline__ void control_loop(const SolveArgs &a, const SM &sm, c
         // ---- P6: step sizes; meanwhile the lane's stage thread of group 0 runs the adjoint sweep (multipliers),
         //      which nothing here depends on.  A least-squares lane (FL_LSQ) gets its flags from that thread.
         bool late = false;
-        if (lane && sm.I(PI_MODE, p) == MODE_STEP) {
-            if (!step_lsq) {
-                ctrl_step(prm, sm, c, p, NG, step_mode);
-                sm.I(PI_FLAGS, p) = FL_LS | (step_mode & (FL_SOC | FL_RESTO));
-                late = true;
-            }
-            sm.I(PI_MODE, p) = MODE_EVAL;
-        }
+        if (lane && sm.I(PI_MODE, p) == MODE_STEP) late = ctrl_step_sizes(prm, sm, c, p, NG, step_lsq, step_mode);
         PROF_MARK(6);
         TRACE_C(7);
         cta_sync<DUAL>(bar_id, bar_count);  // B7
@@ -262,92 +244,38 @@ __global__ void __launch_bounds__(NMPC_MAX_THREADS(SPT, CPB), 1) nmpc_solve_kern
             TRACE_S(0);
             if (!__syncthreads_or(0)) break;   // B2 (vote)
             TRACE_S(1);
-            // ---- P3a: start the lane's next problem (the accepted step was applied and a finished problem flushed
-            //      before the vote, while the control thread fetched the next problems)
-            if (mine) {
-                const int fl = sm.I(PI_FLAGS, p);
-                const int idx = sm.I(PI_NEXT, p);
-                if (idx >= 0) {
-                    double s6[6];
-                    stage_inputs<NC>(sm, p, s6, cf);
-                    if (WARM && (fl & FL_WARM)) {
-#pragma unroll
-                        for (int j = 0; j < SPT; j++)
-                            if (k0 + j < N) stage_init_warm<RATE>(prm, sm, r[j], k0 + j, p, s6, cf, a.warm_in, (size_t)batch, (size_t)idx);
-                    } else {
-#pragma unroll
-                        for (int j = 0; j < SPT; j++)
-                            if (k0 + j < N) stage_init<RATE>(prm, sm, r[j], k0 + j, p, s6, cf);
-                    }
-                } else if ((fl & (FL_SOC | FL_APPLY)) == FL_SOC && sm.I(PI_MODE, p) == MODE_NEWTON) {
-                    // second-order correction: the next right-hand side from the rejected trial point, before the
-                    // coefficients of any stage overwrite the step slots
-#pragma unroll
-                    for (int j = 0; j < SPT; j++)
-                        if (k0 + j < N) stage_soc_rhs<NC>(prm, sm, r[j], k0 + j, p, cf);
-                }
-            }
+            // ---- P3a: start the lane's next problem, or the right-hand side of a second-order correction (the accepted
+            //      step was applied and a finished problem flushed before the vote, while the control thread fetched the
+            //      next problems)
+            if (mine) stages_init<SPT, WARM, RATE, NC>(prm, sm, r, cf, k0, p, a, N, batch);
             TRACE_S(2);
             __syncthreads();  // B3
             TRACE_S(3);
             // ---- P3b: Newton-system coefficients
-            if (mine) {
-                if (sm.I(PI_MODE, p) == MODE_NEWTON) {
-                    const int lsq = sys_kind(sm.I(PI_FLAGS, p)), soc = sm.I(PI_FLAGS, p) & FL_SOC;
-#pragma unroll
-                    for (int j = 0; j < SPT; j++)
-                        if (k0 + j < N) stage_coeffs<RATE, NC>(prm, sm, r[j], k0 + j, p, lsq, cf, soc);
-                }
-            }
+            if (mine) stages_coeffs<SPT, RATE, NC>(prm, sm, r, cf, k0, p, N);
             TRACE_S(4);
             __syncthreads();  // B4
             // ---- P4: control
             __syncthreads();  // B5
             TRACE_S(5);
             // ---- P5: step-dependent work
-            const bool stepping = mine && sm.I(PI_MODE, p) == MODE_STEP;     // (sampled before B6: the control thread
-            const int step_kind = stepping ? sys_kind(sm.I(PI_FLAGS, p)) : 0;  //  rewrites mode and flags in P6)
-            const int step_lsq = step_kind == 1;
-            if (stepping) {
-                const int lsq = step_kind;
-                const HessDiag hd = hess_diag(prm, sm.P(PS_SF, p), sm.P(PS_DW, p), lsq);
-                StepPart acc;
-                part_reset(acc);
-                double gk[SPT][6];
-#pragma unroll
-                for (int j = 0; j < SPT; j++)
-                    if (k0 + j < N) stage_step<RATE, NC>(prm, sm, r[j], k0 + j, p, hd, lsq, acc, gk[j], cf);
-#pragma unroll
-                for (int j = 0; j < SPT; j++)
-                    if (k0 + j < N)
-                        for (int q = 0; q < 6; q++) sm.at(k0 + j, W_0 + q, p) = gk[j][q];
-                part_store(sm, g, p, acc);
-            }
+            StepPart sp;
+            part_reset(sp);
+            const int step_kind = mine ? stages_step<SPT, RATE, NC>(prm, sm, r, cf, k0, p, N, sp) : -1;
+            if (step_kind >= 0) part_store(sm, g, p, sp);
             TRACE_S(6);
             __syncthreads();  // B6
             // ---- P6: the control thread sets the step sizes; a stage thread of lane p runs its adjoint sweep
             // (lanes 0..15 on the thread of group 0, lanes 16..31 on that of group 1: a 64-bit shared-memory access of
             //  16 lanes is one wavefront, and the two half-warps sit on different sub-partitions)
-            if (g == ((NG >= 2) ? (p >> 4) : 0) && stepping) {
-                const int big = adjoint_sweep(prm, sm, p);
-                if (step_lsq) sm.I(PI_FLAGS, p) = FL_ADOPT | ctrl_lsq_finish(prm, sm, p, big);
-            }
+            if (g == ((NG >= 2) ? (p >> 4) : 0) && step_kind >= 0) stage_adjoint(prm, sm, p, step_kind);
             __syncthreads();  // B7
             TRACE_S(7);
             // ---- P1: evaluate
-            if (mine && sm.I(PI_MODE, p) == MODE_EVAL) {
-                const int fl = sm.I(PI_FLAGS, p);
-                EvalPart acc;
-                part_reset(acc);
-                if (fl & FL_ADOPT) {
-#pragma unroll
-                    for (int j = 0; j < SPT; j++)
-                        if (k0 + j < N) stage_adopt(prm, sm, k0 + j, p, fl);
-                }
-#pragma unroll
-                for (int j = 0; j < SPT; j++)
-                    if (k0 + j < N) stage_eval<RATE, NC>(prm, sm, r[j], k0 + j, p, fl, acc, cf);
-                part_store(sm, g, p, acc);
+            if (mine) {
+                EvalPart ep;
+                part_reset(ep);
+                if (stages_eval<SPT, RATE, NC>(prm, sm, r, cf, k0, p, N, ep)) part_store(sm, g, p, ep);
             }
             TRACE_S(8);
             __syncthreads();  // B1
@@ -356,19 +284,7 @@ __global__ void __launch_bounds__(NMPC_MAX_THREADS(SPT, CPB), 1) nmpc_solve_kern
             __syncthreads();  // B1b
             // ---- P3a0: apply the accepted step, flush a finished problem -- while the control thread refills the
             //      lanes (neither touches what the other reads: the step to apply was copied to PS_AP_* in P2)
-            if (mine) {
-                const int fl = sm.I(PI_FLAGS, p);
-                if (fl & FL_APPLY) {
-#pragma unroll
-                    for (int j = 0; j < SPT; j++)
-                        if (k0 + j < N) stage_apply<RATE>(prm, sm, r[j], k0 + j, p);
-                }
-                if (fl & FL_FLUSH) {
-#pragma unroll
-                    for (int j = 0; j < SPT; j++)
-                        if (k0 + j < N) stage_flush(prm, sm, r[j], k0 + j, p, a, N, batch);
-                }
-            }
+            if (mine) stages_apply<SPT, RATE>(prm, sm, r, k0, p, a, N, batch);
         }
     }
 }

@@ -94,11 +94,7 @@ __global__ void __launch_bounds__(384, 1) nmpc_solve_kernel_dual(const SolveArgs
             if (started & (1 << G)) {
                 named_sync(bid, bar_count);   // B1b
                 // ---- P3a0: apply the accepted step, flush a finished problem (the control warp refills meanwhile)
-                if (mine) {
-                    const int fl = sm.I(PI_FLAGS, p);
-                    if (fl & FL_APPLY) stage_apply<RATE>(prm, sm, r, k, p);
-                    if (fl & FL_FLUSH) stage_flush(prm, sm, r, k, p, a, N, batch);
-                }
+                if (mine) stages_apply<1, RATE>(prm, sm, &r, k, p, a, N, batch);
             }
             asm volatile("" ::: "memory");
             if (!named_vote(0, bid, bar_count)) {      // B2 (vote): the group has run out of work
@@ -106,24 +102,10 @@ __global__ void __launch_bounds__(384, 1) nmpc_solve_kernel_dual(const SolveArgs
             } else {
                 started |= 1 << G;
                 // ---- P3a: start the lane's next problem / right-hand side of a second-order correction
-                if (mine) {
-                    const int fl = sm.I(PI_FLAGS, p);
-                    const int idx = sm.I(PI_NEXT, p);
-                    if (idx >= 0) {
-                        double s6[6];
-                        stage_inputs<NC>(sm, p, s6, cf);
-                        if (WARM && (fl & FL_WARM)) stage_init_warm<RATE>(prm, sm, r, k, p, s6, cf, a.warm_in, (size_t)batch, (size_t)idx);
-                        else stage_init<RATE>(prm, sm, r, k, p, s6, cf);
-                    } else if ((fl & (FL_SOC | FL_APPLY)) == FL_SOC && sm.I(PI_MODE, p) == MODE_NEWTON) {
-                        stage_soc_rhs<NC>(prm, sm, r, k, p, cf);
-                    }
-                }
+                if (mine) stages_init<1, WARM, RATE, NC>(prm, sm, &r, cf, k, p, a, N, batch);
                 named_sync(bid, bar_count);   // B3
                 // ---- P3b: Newton-system coefficients
-                if (mine && sm.I(PI_MODE, p) == MODE_NEWTON) {
-                    const int lsq = sys_kind(sm.I(PI_FLAGS, p)), soc = sm.I(PI_FLAGS, p) & FL_SOC;
-                    stage_coeffs<RATE, NC>(prm, sm, r, k, p, lsq, cf, soc);
-                }
+                if (mine) stages_coeffs<1, RATE, NC>(prm, sm, &r, cf, k, p, N);
                 named_sync(bid, bar_count);   // B4: the group's control warp starts its sweeps
             }
         }
@@ -141,41 +123,21 @@ __global__ void __launch_bounds__(384, 1) nmpc_solve_kernel_dual(const SolveArgs
             const bool mine = mine_k && p < PB;
             named_sync(bid, bar_count);       // B5: the sweeps are done
             // ---- P5: step-dependent work
-            const bool stepping = mine && sm.I(PI_MODE, p) == MODE_STEP;       // (sampled before B6: the control thread
-            const int step_kind = stepping ? sys_kind(sm.I(PI_FLAGS, p)) : 0;  //  rewrites mode and flags in P6)
-            const int step_lsq = step_kind == 1;
-            {
-                StepPart acc;
-                part_reset(acc);
-                if (stepping) {
-                    const HessDiag hd = hess_diag(prm, sm.P(PS_SF, p), sm.P(PS_DW, p), step_kind);
-                    double gk[6];
-                    stage_step<RATE, NC>(prm, sm, r, k, p, hd, step_kind, acc, gk, cf);
-                    for (int q = 0; q < 6; q++) sm.at(k, W_0 + q, p) = gk[q];
-                }
-                part_pair(acc);
-                if (stepping && lower) part_store(sm, g, p, acc);
-            }
+            StepPart sp;
+            part_reset(sp);
+            const int step_kind = mine ? stages_step<1, RATE, NC>(prm, sm, &r, cf, k, p, N, sp) : -1;
+            part_pair(sp);
+            if (step_kind >= 0 && lower) part_store(sm, g, p, sp);
             named_sync(bid, bar_count);       // B6
             // ---- P6: the control thread sets the step sizes; the lane's stage-0 thread runs the adjoint sweep
-            if (k == 0 && stepping) {
-                const int big = adjoint_sweep(prm, sm, p);
-                if (step_lsq) sm.I(PI_FLAGS, p) = FL_ADOPT | ctrl_lsq_finish(prm, sm, p, big);
-            }
+            if (k == 0 && step_kind >= 0) stage_adjoint(prm, sm, p, step_kind);
             named_sync(bid, bar_count);       // B7
             // ---- P1: evaluate
-            {
-                EvalPart acc;
-                part_reset(acc);
-                const bool ev = mine && sm.I(PI_MODE, p) == MODE_EVAL;
-                if (ev) {
-                    const int fl = sm.I(PI_FLAGS, p);
-                    if (fl & FL_ADOPT) stage_adopt(prm, sm, k, p, fl);
-                    stage_eval<RATE, NC>(prm, sm, r, k, p, fl, acc, cf);
-                }
-                part_pair(acc);
-                if (ev && lower) part_store(sm, g, p, acc);
-            }
+            EvalPart ep;
+            part_reset(ep);
+            const bool ev = mine && stages_eval<1, RATE, NC>(prm, sm, &r, cf, k, p, N, ep);
+            part_pair(ep);
+            if (ev && lower) part_store(sm, g, p, ep);
             named_sync(bid, bar_count);       // B1: the control warp decides
         }
     }

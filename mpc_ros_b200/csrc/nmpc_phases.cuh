@@ -1795,4 +1795,182 @@ MPC_HD void stage_flush(const Params &prm, const SM &sm, const StageRegs &r, int
     }
 }
 
+// ---------------------------------------------------------------- the phases of one lane
+// What a lane does in each phase, written once for both kernels and the host emulator; the callers keep their own barriers
+// and loops.  The stage side works on one thread's run of stages k0 .. k0+S-1 of lane p (stages >= N are skipped), with the
+// run's registers in r[0 .. S-1] and the lane's path polynomial in cf.  The P5 and P1 helpers accumulate partial sums into
+// the caller's `acc` and leave storing them to the caller: the dual-group kernel first combines them across the two halves
+// of a warp.  As above, N, batch, k0 and p come from the caller.
+
+// P3a, stage side: a lane taking over a new problem (PI_NEXT) initialises the run, from the warm-start record with FL_WARM;
+// a lane about to solve a second-order correction computes its right-hand side from the rejected trial point, before the
+// coefficients of any stage overwrite the step slots.
+template <int S, bool WARM, bool RATE, int NC, class SM>
+MPC_HD void stages_init(const Params &prm, const SM &sm, StageRegs *r, double *cf, int k0, int p, const SolveArgs &a,
+                        const int N, const int batch)
+{
+    const int fl = sm.I(PI_FLAGS, p);
+    const int idx = sm.I(PI_NEXT, p);
+    if (idx >= 0) {
+        // (the polynomial goes to cf last: stored through cf before the initialisation, it changes the register
+        //  allocation of the kernels whose lane count is a run-time value)
+        double s6[6], c[NC];
+        stage_inputs<NC>(sm, p, s6, c);
+        if (WARM && (fl & FL_WARM)) {
+#pragma unroll
+            for (int j = 0; j < S; j++)
+                if (k0 + j < N) stage_init_warm<RATE>(prm, sm, r[j], k0 + j, p, s6, c, a.warm_in, (size_t)batch, (size_t)idx);
+        } else {
+#pragma unroll
+            for (int j = 0; j < S; j++)
+                if (k0 + j < N) stage_init<RATE>(prm, sm, r[j], k0 + j, p, s6, c);
+        }
+#pragma unroll
+        for (int i = 0; i < NC; i++) cf[i] = c[i];
+    } else if ((fl & (FL_SOC | FL_APPLY)) == FL_SOC && sm.I(PI_MODE, p) == MODE_NEWTON) {
+#pragma unroll
+        for (int j = 0; j < S; j++)
+            if (k0 + j < N) stage_soc_rhs<NC>(prm, sm, r[j], k0 + j, p, cf);
+    }
+}
+
+// P3a, control side, after the stage side: the flags it consumed are cleared (FL_SOC next to FL_APPLY: the applied step
+// was a correction), and the lane's next problem becomes its problem.
+template <class SM>
+MPC_HD void ctrl_handover(const SM &sm, int p)
+{
+    const int f0 = sm.I(PI_FLAGS, p);
+    sm.I(PI_FLAGS, p) = f0 & ~(FL_APPLY | FL_FLUSH | FL_WARM | ((f0 & FL_APPLY) ? FL_SOC : 0));
+    if (sm.I(PI_NEXT, p) >= 0) { sm.I(PI_PROB, p) = sm.I(PI_NEXT, p); sm.I(PI_NEXT, p) = -1; }
+}
+
+// P3b, stage side: the Newton-system coefficients of a lane in MODE_NEWTON.
+template <int S, bool RATE, int NC, class SM>
+MPC_HD void stages_coeffs(const Params &prm, const SM &sm, StageRegs *r, const double *cf, int k0, int p, const int N)
+{
+    if (sm.I(PI_MODE, p) == MODE_NEWTON) {
+        const int lsq = sys_kind(sm.I(PI_FLAGS, p)), soc = sm.I(PI_FLAGS, p) & FL_SOC;
+#pragma unroll
+        for (int j = 0; j < S; j++)
+            if (k0 + j < N) stage_coeffs<RATE, NC>(prm, sm, r[j], k0 + j, p, lsq, cf, soc);
+    }
+}
+
+// P4, control side, lane in MODE_NEWTON, in two parts (the kernels mark the profile between them).  The first samples the
+// system to solve (lsq: its sys_kind; mode: its FL_SOC / FL_RESUME / FL_RESTO, kept for P6, where the adjoint sweep's
+// thread may rewrite PI_FLAGS), forms the regularised Hessian diagonal and runs the backward sweep.
+struct NewtonSys { int lsq, mode, ok; double dw; HessDiag hd; };
+template <bool RATE, class SM>
+MPC_HD NewtonSys ctrl_newton_backward(const Params &prm, const SM &sm, int p)
+{
+    NewtonSys s;
+    s.lsq = sys_kind(sm.I(PI_FLAGS, p));
+    s.mode = sm.I(PI_FLAGS, p) & (FL_SOC | FL_RESUME | FL_RESTO);
+    s.dw = sm.P(PS_DW, p);
+    s.hd = hess_diag(prm, sm.P(PS_SF, p), s.dw, s.lsq);
+    s.ok = riccati_backward<RATE>(prm, sm, p, s.hd);
+    return s;
+}
+// The second runs the forward sweep, after which the lane steps.  If the factorisation had the wrong inertia, the lane
+// stays in MODE_NEWTON with the next regularisation (its coefficients are rewritten next cycle), or fails with status 10
+// when that would exceed NMPC_DW_MAX; either way it returns 1 (an inertia-correction retry).
+template <bool RATE, class SM>
+MPC_HD int ctrl_newton_forward(const Params &prm, const SM &sm, Ctrl &c, int p, const NewtonSys &s)
+{
+    if (s.ok || s.lsq) {
+        riccati_forward<RATE>(prm, sm, p, s.hd);
+        if (s.dw > 0.0) c.dw_last = s.dw;
+        sm.I(PI_MODE, p) = MODE_STEP;
+        return 0;
+    }
+    const double nd = next_dw(c, s.dw);
+    if (nd > NMPC_DW_MAX) { c.status = 10; sm.I(PI_MODE, p) = MODE_FAIL; }
+    else sm.P(PS_DW, p) = nd;
+    return 1;
+}
+
+// P5, stage side, lane in MODE_STEP: the step-dependent work of the run, then its g_k into W_0..W_5.  Returns the sys_kind
+// of the system stepped, or -1 when the lane is not stepping.  The kernels sample it before B6 for P6, since the control
+// thread rewrites the lane's mode and flags there.  (One return value chosen up front: with an early return the
+// dual-group kernel keeps a different set of values live across B6.)
+template <int S, bool RATE, int NC, class SM>
+MPC_HD int stages_step(const Params &prm, const SM &sm, StageRegs *r, const double *cf, int k0, int p, const int N, StepPart &acc)
+{
+    const bool stepping = sm.I(PI_MODE, p) == MODE_STEP;
+    const int kind = stepping ? sys_kind(sm.I(PI_FLAGS, p)) : -1;
+    if (stepping) {
+        const HessDiag hd = hess_diag(prm, sm.P(PS_SF, p), sm.P(PS_DW, p), kind);
+        double gk[S][6];
+#pragma unroll
+        for (int j = 0; j < S; j++)
+            if (k0 + j < N) stage_step<RATE, NC>(prm, sm, r[j], k0 + j, p, hd, kind, acc, gk[j], cf);
+#pragma unroll
+        for (int j = 0; j < S; j++)
+            if (k0 + j < N)
+                for (int q = 0; q < 6; q++) sm.at(k0 + j, W_0 + q, p) = gk[j][q];
+    }
+    return kind;
+}
+
+// P6, stage side, lane stepping a system of sys_kind `kind` (stages_step): the adjoint sweep; after the least-squares start
+// it also sets the lane's flags for P1, which adopts or zeroes the multipliers.
+template <class SM>
+MPC_HD void stage_adjoint(const Params &prm, const SM &sm, int p, int kind)
+{
+    const int big = adjoint_sweep(prm, sm, p);
+    if (kind == 1) sm.I(PI_FLAGS, p) = FL_ADOPT | ctrl_lsq_finish(prm, sm, p, big);
+}
+
+// P6, control side, lane in MODE_STEP (lsq: the system was the least-squares start; mode: as sampled in P4): the step sizes
+// and the line-search flags, except after the least-squares start, whose flags stage_adjoint sets.  The lane evaluates in
+// P1.  Returns 1 when ctrl_step ran: ctrl_step_late is then due before P2.
+template <class SM>
+MPC_HD int ctrl_step_sizes(const Params &prm, const SM &sm, Ctrl &c, int p, int NG, int lsq, int mode)
+{
+    int late = 0;
+    if (!lsq) {
+        ctrl_step(prm, sm, c, p, NG, mode);
+        sm.I(PI_FLAGS, p) = FL_LS | (mode & (FL_SOC | FL_RESTO));
+        late = 1;
+    }
+    sm.I(PI_MODE, p) = MODE_EVAL;
+    return late;
+}
+
+// P1, stage side, lane in MODE_EVAL: adopts the least-squares multipliers first (FL_ADOPT), then evaluates the run into acc.
+// Returns whether the lane evaluated.
+template <int S, bool RATE, int NC, class SM>
+MPC_HD bool stages_eval(const Params &prm, const SM &sm, StageRegs *r, const double *cf, int k0, int p, const int N, EvalPart &acc)
+{
+    if (sm.I(PI_MODE, p) != MODE_EVAL) return false;
+    const int fl = sm.I(PI_FLAGS, p);
+    if (fl & FL_ADOPT) {
+#pragma unroll
+        for (int j = 0; j < S; j++)
+            if (k0 + j < N) stage_adopt(prm, sm, k0 + j, p, fl);
+    }
+#pragma unroll
+    for (int j = 0; j < S; j++)
+        if (k0 + j < N) stage_eval<RATE, NC>(prm, sm, r[j], k0 + j, p, fl, acc, cf);
+    return true;
+}
+
+// P3a0, stage side: applies the step P2 accepted (FL_APPLY) and writes a finished problem out (FL_FLUSH).
+template <int S, bool RATE, class SM>
+MPC_HD void stages_apply(const Params &prm, const SM &sm, StageRegs *r, int k0, int p, const SolveArgs &a, const int N,
+                         const int batch)
+{
+    const int fl = sm.I(PI_FLAGS, p);
+    if (fl & FL_APPLY) {
+#pragma unroll
+        for (int j = 0; j < S; j++)
+            if (k0 + j < N) stage_apply<RATE>(prm, sm, r[j], k0 + j, p);
+    }
+    if (fl & FL_FLUSH) {
+#pragma unroll
+        for (int j = 0; j < S; j++)
+            if (k0 + j < N) stage_flush(prm, sm, r[j], k0 + j, p, a, N, batch);
+    }
+}
+
 }  // namespace nmpc

@@ -1,14 +1,16 @@
 // tests/emu/nmpc_emu.cpp -- TEST INFRASTRUCTURE, NOT PRODUCT CODE.
 //
-// Runs the solver's phase functions (mpc_ros_b200/csrc/nmpc_phases.cuh, the code the CUDA
-// kernel executes: the arithmetic, the per-lane state machine, the start of a problem in a lane and
-// the write-out of its results) sequentially on the host, one emulated CTA of PB lanes at a time, with
-// the kernel's cycle / barrier structure (nmpc_kernel.cuh) turned into plain loops.  (The kernel's
-// work queue is not emulated: lanes get their problems statically; results do not depend on the
-// lane, which the tests check.)  It exists so that the
-// solver LOGIC can be checked against the oracle in the CPU-only test tier (this container has no
-// GPU).  It is built only by tests/ into tests/emu/libnmpc_emu.so, is never linked into
-// libmpc_b200.so, and nothing in the product path can reach it.
+// Runs the solver's phase functions (mpc_ros_b200/csrc/nmpc_phases.cuh, the code both CUDA kernels
+// execute: the arithmetic, what each lane does in each phase, the per-lane state machine, the start of
+// a problem in a lane and the write-out of its results) sequentially on the host, one emulated CTA of
+// PB lanes at a time.  What is the emulator's own is the driver: the kernel's cycle (nmpc_kernel.cuh)
+// as one loop per phase over the lanes and their stage groups of SPT stages, in the kernel's phase
+// order and in ascending groups, in place of the barriers; the P2 loop; and the counters.  (The
+// kernel's work queue is not emulated: lanes get their problems statically, and there is no warm-start
+// input; results do not depend on the lane, which the tests check.)  It exists so that the solver
+// LOGIC can be checked against the oracle in the CPU-only test tier (this container has no GPU).  It
+// is built only by tests/ into tests/emu/libnmpc_emu.so, is never linked into libmpc_b200.so, and
+// nothing in the product path can reach it.
 #include "../../mpc_ros_b200/csrc/nmpc_phases.cuh"
 #include <vector>
 #include <cstring>
@@ -58,11 +60,13 @@ static int emu_run(const SolveArgs &a, int *n_reg)
     const int NS = RATE ? NSLOTS_RATE : NSLOTS;
     std::vector<double> mem(smem_bytes(N, NG, PB, NS) / sizeof(double) + 8);
     SmemT<0, RATE ? NSLOTS_RATE : NSLOTS> sm; sm.PB = PB; sm.carve(mem.data(), N, NG);
-    std::vector<StageRegs> regs((size_t)N * PB);
+    std::vector<StageRegs> regs((size_t)PB * N);   // [lane][stage]: the run of a stage group is contiguous
     std::vector<double> cfs((size_t)NC * PB);
     std::vector<Ctrl> ctrl(PB);
-    std::vector<int> nreg(PB);
-#define REG(k, p) regs[(size_t)(k) * PB + (p)]
+    std::vector<NewtonSys> sys(PB);                // P4 -> P6, as the control thread keeps it
+    std::vector<int> nreg(PB), step_kind(PB);      // step_kind: P5 -> P6, as the stage threads keep it
+    // the arguments of the stage helpers for group g of lane p: its run of registers, the path polynomial, k0 and p
+#define RUN(p, g) &regs[(size_t)(p) * N + (g) * SPT], &cfs[(size_t)NC * (p)], (g) * SPT, (p)
 
     for (int base = 0; base < batch; base += PB) {
         const int np = (batch - base < PB) ? batch - base : PB;
@@ -80,90 +84,38 @@ static int emu_run(const SolveArgs &a, int *n_reg)
             if (!active) break;
             for (int p = 0; p < np; p++) g_lane_cycles += (sm.I(PI_MODE, p) != MODE_IDLE);
             // ---- P3a
-            for (int p = 0; p < np; p++) {
-                const int fl = sm.I(PI_FLAGS, p);
-                if (fl & FL_APPLY) for (int k = 0; k < N; k++) stage_apply<RATE>(prm, sm, REG(k, p), k, p);
-                if (fl & FL_FLUSH) for (int k = 0; k < N; k++) stage_flush(prm, sm, REG(k, p), k, p, a, N, batch);
-                if (sm.I(PI_NEXT, p) >= 0) {
-                    double s6[6];
-                    stage_inputs<NC>(sm, p, s6, &cfs[(size_t)NC * p]);
-                    for (int k = 0; k < N; k++) stage_init<RATE>(prm, sm, REG(k, p), k, p, s6, &cfs[(size_t)NC * p]);
-                }
-            }
-            // second-order correction: next right-hand side from the rejected trial point, before any stage's coefficients
-            // overwrite the step slots
             for (int p = 0; p < np; p++)
-                if (sm.I(PI_MODE, p) == MODE_NEWTON && (sm.I(PI_FLAGS, p) & (FL_SOC | FL_APPLY)) == FL_SOC)
-                    for (int k = 0; k < N; k++) stage_soc_rhs<NC>(prm, sm, REG(k, p), k, p, &cfs[(size_t)NC * p]);
-            for (int p = 0; p < np; p++) {
-                if (sm.I(PI_FLAGS, p) & FL_APPLY) sm.I(PI_FLAGS, p) &= ~FL_SOC;
-                sm.I(PI_FLAGS, p) &= ~(FL_APPLY | FL_FLUSH);
-                if (sm.I(PI_NEXT, p) >= 0) { sm.I(PI_PROB, p) = sm.I(PI_NEXT, p); sm.I(PI_NEXT, p) = -1; }
-            }
+                for (int g = 0; g < NG; g++) stages_init<SPT, false, RATE, NC>(prm, sm, RUN(p, g), a, N, batch);
+            for (int p = 0; p < np; p++) ctrl_handover(sm, p);
             // ---- P3b
             for (int p = 0; p < np; p++)
-                if (sm.I(PI_MODE, p) == MODE_NEWTON)
-                    for (int k = 0; k < N; k++) stage_coeffs<RATE, NC>(prm, sm, REG(k, p), k, p, sys_kind(sm.I(PI_FLAGS, p)), &cfs[(size_t)NC * p], sm.I(PI_FLAGS, p) & FL_SOC);
+                for (int g = 0; g < NG; g++) stages_coeffs<SPT, RATE, NC>(prm, sm, RUN(p, g), N);
             // ---- P4
-            for (int p = 0; p < np; p++) {
-                if (sm.I(PI_MODE, p) != MODE_NEWTON) continue;
-                Ctrl &c = ctrl[p];
-                const int lsq = sys_kind(sm.I(PI_FLAGS, p));
-                const double dw = sm.P(PS_DW, p);
-                const HessDiag hd = hess_diag(prm, sm.P(PS_SF, p), dw, lsq);
-                if (riccati_backward<RATE>(prm, sm, p, hd) || lsq) {
-                    riccati_forward<RATE>(prm, sm, p, hd);
-                    if (dw > 0.0) c.dw_last = dw;
-                    sm.I(PI_MODE, p) = MODE_STEP;
-                } else {
-                    const double nd = next_dw(c, dw);
-                    nreg[p]++;
-                    if (nd > NMPC_DW_MAX) { c.status = 10; sm.I(PI_MODE, p) = MODE_FAIL; }
-                    else sm.P(PS_DW, p) = nd;
+            for (int p = 0; p < np; p++)
+                if (sm.I(PI_MODE, p) == MODE_NEWTON) {
+                    sys[p] = ctrl_newton_backward<RATE>(prm, sm, p);
+                    nreg[p] += ctrl_newton_forward<RATE>(prm, sm, ctrl[p], p, sys[p]);
                 }
-            }
             // ---- P5
-            for (int p = 0; p < np; p++) {
-                if (sm.I(PI_MODE, p) != MODE_STEP) continue;
-                const int lsq = sys_kind(sm.I(PI_FLAGS, p));
-                const HessDiag hd = hess_diag(prm, sm.P(PS_SF, p), sm.P(PS_DW, p), lsq);
+            for (int p = 0; p < np; p++)
                 for (int g = 0; g < NG; g++) {
                     StepPart acc; part_reset(acc);
-                    double gk[SPT][6];
-                    for (int k = g * SPT; k < g * SPT + SPT && k < N; k++) stage_step<RATE, NC>(prm, sm, REG(k, p), k, p, hd, lsq, acc, gk[k - g * SPT], &cfs[(size_t)NC * p]);
-                    for (int k = g * SPT; k < g * SPT + SPT && k < N; k++)
-                        for (int q = 0; q < 6; q++) sm.at(k, W_0 + q, p) = gk[k - g * SPT][q];
-                    part_store(sm, g, p, acc);
+                    step_kind[p] = stages_step<SPT, RATE, NC>(prm, sm, RUN(p, g), N, acc);
+                    if (step_kind[p] >= 0) part_store(sm, g, p, acc);
                 }
-            }
             // ---- P6
             for (int p = 0; p < np; p++) {
-                if (sm.I(PI_MODE, p) != MODE_STEP) continue;
-                const int big = adjoint_sweep(prm, sm, p);
-                if (sm.I(PI_FLAGS, p) & FL_LSQ) {
-                    const int keep = ctrl_lsq_finish(prm, sm, p, big);
-                    sm.I(PI_FLAGS, p) = FL_ADOPT | keep;
-                } else {
-                    const int mode = sm.I(PI_FLAGS, p) & (FL_SOC | FL_RESUME | FL_RESTO);
-                    ctrl_step(prm, sm, ctrl[p], p, NG, mode);
+                if (step_kind[p] >= 0) stage_adjoint(prm, sm, p, step_kind[p]);
+                if (sm.I(PI_MODE, p) == MODE_STEP && ctrl_step_sizes(prm, sm, ctrl[p], p, NG, sys[p].lsq == 1, sys[p].mode))
                     ctrl_step_late(ctrl[p]);
-                    sm.I(PI_FLAGS, p) = FL_LS | (mode & (FL_SOC | FL_RESTO));
-                }
-                sm.I(PI_MODE, p) = MODE_EVAL;
             }
-            // ---- P1
-            for (int p = 0; p < np; p++) {
-                if (sm.I(PI_MODE, p) != MODE_EVAL) continue;
-                const int fl = sm.I(PI_FLAGS, p);
-                // all stages read their neighbours' slots before FL_ADOPT overwrites the L slots of a stage:
-                // stage k writes only its own L slots and reads lambda^+ of stage k-1 from W, as in the kernel
-                if (fl & FL_ADOPT) for (int k = 0; k < N; k++) stage_adopt(prm, sm, k, p, fl);
+            // ---- P1 (each group adopts before it evaluates, as in the kernels: after an adoption, an evaluation uses the
+            //      L slots of its own stages only)
+            for (int p = 0; p < np; p++)
                 for (int g = 0; g < NG; g++) {
                     EvalPart acc; part_reset(acc);
-                    for (int k = g * SPT; k < g * SPT + SPT && k < N; k++) stage_eval<RATE, NC>(prm, sm, REG(k, p), k, p, fl, acc, &cfs[(size_t)NC * p]);
-                    part_store(sm, g, p, acc);
+                    if (stages_eval<SPT, RATE, NC>(prm, sm, RUN(p, g), N, acc)) part_store(sm, g, p, acc);
                 }
-            }
             // ---- P2
             for (int p = 0; p < np; p++) {
                 Ctrl &c = ctrl[p];
@@ -183,8 +135,12 @@ static int emu_run(const SolveArgs &a, int *n_reg)
                     ctrl_finish(prm, sm, c, p, a, N, batch);
                 }
             }
+            // ---- P3a0
+            for (int p = 0; p < np; p++)
+                for (int g = 0; g < NG; g++) stages_apply<SPT, RATE>(prm, sm, &regs[(size_t)p * N + g * SPT], g * SPT, p, a, N, batch);
         }
     }
+#undef RUN
     return 0;
 }
 
