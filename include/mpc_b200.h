@@ -143,7 +143,13 @@ int32_t mpc_b200_warm_size(int32_t mpc_steps);
  *                        rewrites REF_V per tick (driving_state.cpp:127-139)
  *   warm_in  warm_size x batch, optional, device or host memory (NULL = the reference's cold start, :288-300):
  *            controls, equality and bound multipliers are taken from it, the states are re-derived
- *            by a roll-out of the model from `state`
+ *            by a roll-out of the model from `state` (the record's state rows are not read).  Controls
+ *            are clipped 1e-3 U inside the relaxed bounds U, so a NaN control is read as U - 1e-3 U;
+ *            z = max(sf z, warm_mu_init / slack), so a NaN bound multiplier is read as the floor and an
+ *            infinite one ends the problem at once with status 11.  A non-finite equality multiplier
+ *            (lambda_0 included) ends it after the start point's evaluation with status 10 and 0
+ *            iterations, as Ipopt's first step would (at mpc_steps = 2, where no multiplier enters a
+ *            Newton system, with status 11 at that evaluation): it is never carried into a status-1 result.
  *   u0       2 x batch   {w_0, throttle_0} = MPC::Solve's return value (:398-401)
  *   pred     3N x batch  mpc_x, mpc_y, mpc_theta (:388-396)
  *   obj      batch       objective value (solution.obj_value, :381), optional

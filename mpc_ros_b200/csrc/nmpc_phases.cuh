@@ -408,10 +408,23 @@ MPC_HD void stage_init_warm(const Params &prm, const SM &sm, StageRegs &r, int k
         sm.at(k, W_10, p) = uw; sm.at(k, W_11, p) = ua;    // for the roll-out
         if (RATE) { sm.at(k, U_W, p) = uw; sm.at(k, U_A, p) = ua; }
         const size_t offl = warm_lam(N), offz = warm_z(N);
-        for (int c = 0; c < 6; c++) sm.at(k, L_X + c, p) = sf * warm[(offl + (size_t)c * N + k + 1) * stride + idx];
+        // A non-finite equality multiplier must not end in a "success": the max of the dual residuals drops a NaN, and only
+        // the x, y and cte components of lambda_{k+1} at a free stage (k >= 1) enter a Newton system, through the Hessian.
+        // bad is +0 when the entries it sums are finite, else NaN (0 * |l|, one term per entry, so that finite entries
+        // cannot overflow).  A non-finite component of lambda_{k+1} is spread over all six, and stage 1 also takes in
+        // lambda_0 and lambda_1, which enter no Newton system: the first Newton step then fails with status 10, as the
+        // oracle's does.  At N = 2 no multiplier enters a Newton system; there stage 0 takes in lambda_0 and lambda_1 and
+        // makes z_L,w NaN, which ends the problem with status 11 at its first evaluation.  Finite records are read
+        // unchanged: l - (+0) is l bit for bit, -0 included, and z_L,w > 0.
+        double bad = 0.0;
+        for (int c = 0; c < 6; c++) bad += 0.0 * fabs(warm[(offl + (size_t)c * N + k + 1) * stride + idx]);
+        if (k == 1 || N == 2)
+            for (int c = 0; c < 6; c++) bad += 0.0 * fabs(warm[(offl + (size_t)c * N) * stride + idx]) + 0.0 * fabs(warm[(offl + (size_t)c * N + 1) * stride + idx]);
+        for (int c = 0; c < 6; c++) sm.at(k, L_X + c, p) = sf * warm[(offl + (size_t)c * N + k + 1) * stride + idx] - bad;
         const int nu = N - 1;
         // multipliers of the control bounds: at least on the central path of the starting mu
         r.zlw = fmax2(sf * warm[(offz + k) * stride + idx], mu / (uw + Uw));
+        if (N == 2) r.zlw += bad;
         r.zla = fmax2(sf * warm[(offz + nu + k) * stride + idx], mu / (ua + Ua));
         r.zuw = fmax2(sf * warm[(offz + 2 * nu + k) * stride + idx], mu / (Uw - uw));
         r.zua = fmax2(sf * warm[(offz + 3 * nu + k) * stride + idx], mu / (Ua - ua));

@@ -203,6 +203,11 @@ static int filter_ok(const filt_entry *flt, int nf, double theta_max, double the
 
 int ipm_solve(const ipm_nlp *nlp, const ipm_options *opt, ipm_result *res)
 {
+    return ipm_solve_from(nlp, opt, NULL, res);
+}
+
+int ipm_solve_from(const ipm_nlp *nlp, const ipm_options *opt, const ipm_start *start, ipm_result *res)
+{
     const double t_start = cpu_now();
     ipm_ws W; memset(&W, 0, sizeof(W));
     ipm_ws *w = &W;
@@ -260,7 +265,7 @@ int ipm_solve(const ipm_nlp *nlp, const ipm_options *opt, ipm_result *res)
 
     int status = IPM_INTERNAL_ERROR;
     int iter = 0;
-    double mu = opt->mu_init;
+    double mu = start ? start->mu0 : opt->mu_init;
     int n_inertia = 0, n_resto = 0;
     double E0 = INFINITY;
 
@@ -304,6 +309,11 @@ int ipm_solve(const ipm_nlp *nlp, const ipm_options *opt, ipm_result *res)
         for (int i = 0; i < m; i++) if (rowmax[i] > gmax) w->sc[i] = gmax / rowmax[i];
         free(rowmax);
     }
+    /* a given start: the scaling stays the cold start's, the iterate is the given one (not pushed) */
+    if (start) {
+        if (start->sf > 0.0) w->sf = start->sf;
+        memcpy(X, start->x0, sizeof(double) * n);
+    }
     for (int i = 0; i < m; i++) {
         w->gl[i] = (glr[i] > -IPM_INF) ? w->sc[i] * glr[i] : -INFINITY;
         w->gu[i] = (gur[i] < IPM_INF) ? w->sc[i] * gur[i] : INFINITY;
@@ -335,6 +345,13 @@ int ipm_solve(const ipm_nlp *nlp, const ipm_options *opt, ipm_result *res)
     w->nbL = w->nbU = 0;
     for (int i = 0; i < N; i++) { w->nbL += w->hasL[i]; w->nbU += w->hasU[i]; }
     for (int i = 0; i < N; i++) { zL[i] = w->hasL[i] ? 1.0 : 0.0; zU[i] = w->hasU[i] ? 1.0 : 0.0; }
+    if (start) {
+        for (int i = 0; i < n; i++) {
+            if (w->hasL[i]) zL[i] = start->zl0[i];
+            if (w->hasU[i]) zU[i] = start->zu0[i];
+        }
+        memcpy(lam, start->lambda0, sizeof(double) * m);
+    }
 
     /* ---- KKT ordering (RCM on the pattern of the augmented system) ---- */
     {
@@ -356,8 +373,8 @@ int ipm_solve(const ipm_nlp *nlp, const ipm_options *opt, ipm_result *res)
     double f;
     if (!ev_fc(w, X, &f, c) || !ev_grad(w, X, gradf) || !ev_jac(w, X)) { status = IPM_INVALID_NUMBER_DETECTED; goto done; }
 
-    /* ---- least-squares multiplier start (W&B eq. (36)) ---- */
-    if (m > 0) {
+    /* ---- least-squares multiplier start (W&B eq. (36)); a given start brings its own ---- */
+    if (m > 0 && !start) {
         for (int i = 0; i < N; i++) Sigma[i] = 1.0;
         kkt_factor(w, Sigma, 0, 0.0, 0.0);
         for (int i = 0; i < N; i++) r1[i] = -(gradf[i] - zL[i] + zU[i]);

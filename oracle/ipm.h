@@ -96,8 +96,25 @@ typedef struct ipm_result {
     double *lambda; /* m */
 } ipm_result;
 
+/* A given starting iterate (warm start).  Multipliers are in the solver's scaled units:
+ * lambda_i = sf * lambda_i(unscaled) / sc_i, z = sf * z(unscaled).  The NLP scaling is the cold solve's:
+ * computed at the NLP's own (pushed) starting point, so a warm solve differs from a cold one in its
+ * starting iterate only; sf > 0 overrides the objective factor.  With a start the solver takes x0 as
+ * given (no bound_push), sets mu = mu0 and tau = max(0.99, 1 - mu0), skips the least-squares
+ * multiplier solve, and uses zL0 / zU0 for the bounds of x (slacks keep z = 1). */
+typedef struct ipm_start {
+    const double *x0;       /* n */
+    const double *lambda0;  /* m */
+    const double *zl0;      /* n */
+    const double *zu0;      /* n */
+    double mu0;
+    double sf;              /* > 0: objective scaling factor; <= 0: computed as for the cold start */
+} ipm_start;
+
 void ipm_default_options(ipm_options *o);
 int ipm_solve(const ipm_nlp *nlp, const ipm_options *opt, ipm_result *res);
+/* start == NULL: ipm_solve */
+int ipm_solve_from(const ipm_nlp *nlp, const ipm_options *opt, const ipm_start *start, ipm_result *res);
 
 #ifdef __cplusplus
 }

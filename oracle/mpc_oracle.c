@@ -253,9 +253,9 @@ static int cb_hstruct(void *u, int *ir, int *jc)
 static int cb_hess(void *u, const double *x, double sigma, const double *lam, double *v)
 { nlp_ctx *c = (nlp_ctx *)u; hess_coo(c->p, c->coeffs, c->ncoef, x, sigma, lam, NULL, NULL, v); return 1; }
 
-int mpc_oracle_solve(const mpc_oracle_params *p, const double *state6, const double *coeffs, int ncoef,
-                     const ipm_options *opt_in, double *u0, double *pred, double *sol, double *lambda,
-                     double *zl, double *zu, mpc_oracle_result *out)
+static int solve_from(const mpc_oracle_params *p, const double *state6, const double *coeffs, int ncoef,
+                      const ipm_options *opt_in, const ipm_start *start, double *u0, double *pred, double *sol,
+                      double *lambda, double *zl, double *zu, mpc_oracle_result *out)
 {
     const int N = p->mpc_steps; LAYOUT(N)
     const int n = mpc_oracle_nvars(N), m = mpc_oracle_ncons(N);
@@ -271,7 +271,7 @@ int mpc_oracle_solve(const mpc_oracle_params *p, const double *state6, const dou
     ipm_result r; memset(&r, 0, sizeof(r));
     double *x = (double *)malloc(sizeof(double) * n);
     r.x = x; r.lambda = lambda; r.zl = zl; r.zu = zu; r.g = NULL;
-    int st = ipm_solve(&nlp, &opt, &r);
+    int st = ipm_solve_from(&nlp, &opt, start, &r);
     if (u0) { u0[0] = x[ws]; u0[1] = x[as]; }                                              /* :399-400 */
     if (pred) for (int i = 0; i < N; i++) { pred[i] = x[xs + i]; pred[N + i] = x[ys + i]; pred[2 * N + i] = x[ts + i]; } /* :391-396 */
     if (sol) memcpy(sol, x, sizeof(double) * n);
@@ -281,6 +281,83 @@ int mpc_oracle_solve(const mpc_oracle_params *p, const double *state6, const dou
         out->n_inertia_corrections = r.n_inertia_corrections; out->n_restorations = r.n_restorations;
     }
     free(x);
+    return st;
+}
+
+int mpc_oracle_solve(const mpc_oracle_params *p, const double *state6, const double *coeffs, int ncoef,
+                     const ipm_options *opt, double *u0, double *pred, double *sol, double *lambda,
+                     double *zl, double *zu, mpc_oracle_result *out)
+{
+    return solve_from(p, state6, coeffs, ncoef, opt, NULL, u0, pred, sol, lambda, zl, zu, out);
+}
+
+int mpc_oracle_solve_warm(const mpc_oracle_params *p, const double *state6, const double *coeffs, int ncoef,
+                          const ipm_options *opt_in, const double *rec, double warm_mu,
+                          double *u0, double *pred, double *sol, double *lambda, double *zl, double *zu,
+                          mpc_oracle_result *out)
+{
+    if (!(p->bound_value >= 1e19)) return -1;      /* the record carries no state-bound multipliers */
+    const int N = p->mpc_steps; LAYOUT(N)
+    const int n = mpc_oracle_nvars(N), m = mpc_oracle_ncons(N), nu = N - 1;
+    const int rl = n, rz = n + m;                   /* record: primal, lambda, zL_w, zL_a, zU_w, zU_a */
+    ipm_options opt;
+    if (opt_in) opt = *opt_in; else ipm_default_options(&opt);
+    double *x = (double *)calloc(n, sizeof(double)), *gr = (double *)malloc(sizeof(double) * n);
+    double *lam = (double *)malloc(sizeof(double) * m);
+    double *zl0 = (double *)calloc(n, sizeof(double)), *zu0 = (double *)calloc(n, sizeof(double));
+
+    /* objective scaling of the cold start (cb_start's point; no state bounds, so nothing is pushed) */
+    const int comp[6] = { xs, ys, ts, vs, cs, es };
+    for (int k = 0; k < 6; k++) x[comp[k]] = state6[k];
+    mpc_oracle_eval_grad(p, coeffs, ncoef, x, gr);
+    double gn = 0.0;
+    for (int i = 0; i < n; i++) gn = fmax(gn, fabs(gr[i]));
+    const double sf = (opt.nlp_scaling_max_gradient > 0.0 && gn > opt.nlp_scaling_max_gradient)
+                      ? opt.nlp_scaling_max_gradient / gn : 1.0;
+
+    /* controls from the record, clipped 1e-3 U inside the relaxed bounds U */
+    const double Uw = p->max_angvel + opt.bound_relax_factor * fmax(1.0, p->max_angvel);
+    const double Ua = p->max_throttle + opt.bound_relax_factor * fmax(1.0, p->max_throttle);
+    for (int k = 0; k < nu; k++) {
+        x[ws + k] = fmax(fmin(rec[ws + k], Uw - 1e-3 * Uw), -Uw + 1e-3 * Uw);
+        x[as + k] = fmax(fmin(rec[as + k], Ua - 1e-3 * Ua), -Ua + 1e-3 * Ua);
+    }
+    /* states: the model rolled out from state6 with those controls, as eval_fg writes the dynamics */
+    for (int i = 0; i < N - 1; i++) {
+        const double x0 = x[xs + i], y0 = x[ys + i], th0 = x[ts + i], v0 = x[vs + i], e0 = x[es + i];
+        const double w0 = x[ws + i], a0 = x[as + i];
+        const double f0 = poly(coeffs, ncoef, x0);
+        x[xs + i + 1] = x0 + v0 * cos(th0) * p->dt;
+        x[ys + i + 1] = y0 + v0 * sin(th0) * p->dt;
+        x[ts + i + 1] = th0 + w0 * p->dt;
+        x[vs + i + 1] = v0 + a0 * p->dt;
+        x[cs + i + 1] = (f0 - y0) + (v0 * sin(e0) * p->dt);
+        x[es + i + 1] = e0 + w0 * p->dt;
+    }
+    /* multipliers in the solver's scaled units, lambda_i = sf lambda_i(record) / sc_i: refused where the cold start
+     * scales a constraint row (sc_i != 1), which the record's rule does not provide for; z at least mu / slack */
+    {
+        const int nnz = mpc_oracle_nnz_jac(N);
+        int *ir = (int *)malloc(sizeof(int) * nnz), *jc = (int *)malloc(sizeof(int) * nnz);
+        double *jv = (double *)malloc(sizeof(double) * nnz), *x_cold = (double *)calloc(n, sizeof(double));
+        for (int k = 0; k < 6; k++) x_cold[comp[k]] = state6[k];
+        jac_coo(p, coeffs, ncoef, x_cold, ir, jc, jv);
+        int scaled = 0;
+        for (int k = 0; k < nnz; k++) scaled |= opt.nlp_scaling_max_gradient > 0.0 && fabs(jv[k]) > opt.nlp_scaling_max_gradient;
+        free(ir); free(jc); free(jv); free(x_cold);
+        if (scaled) { free(x); free(gr); free(lam); free(zl0); free(zu0); return -1; }
+    }
+    for (int i = 0; i < m; i++) lam[i] = sf * rec[rl + i];
+    for (int k = 0; k < nu; k++) {
+        const double w = x[ws + k], a = x[as + k];
+        zl0[ws + k] = fmax(sf * rec[rz + k], warm_mu / (w + Uw));
+        zl0[as + k] = fmax(sf * rec[rz + nu + k], warm_mu / (a + Ua));
+        zu0[ws + k] = fmax(sf * rec[rz + 2 * nu + k], warm_mu / (Uw - w));
+        zu0[as + k] = fmax(sf * rec[rz + 3 * nu + k], warm_mu / (Ua - a));
+    }
+    ipm_start start = { x, lam, zl0, zu0, warm_mu, sf };
+    const int st = solve_from(p, state6, coeffs, ncoef, &opt, &start, u0, pred, sol, lambda, zl, zu, out);
+    free(x); free(gr); free(lam); free(zl0); free(zu0);
     return st;
 }
 

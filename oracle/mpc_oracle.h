@@ -63,6 +63,19 @@ int mpc_oracle_solve(const mpc_oracle_params *p, const double *state6, const dou
                      double *u0, double *pred, double *sol, double *lambda, double *zl, double *zu,
                      mpc_oracle_result *res);
 
+/* The same solve from a warm-start record in the layout of the GPU path's mpc_b200_warm_size (no reference
+ * counterpart: primal 8N-2, lambda 6N, then zL_w, zL_a, zU_w, zU_a of N-1 each; multipliers unscaled).
+ * Restates the record's rule: controls from the record clipped 1e-3 U inside the relaxed bounds U; states
+ * rolled out from state6 with this file's model (the record's states are ignored); lambda (lambda_0
+ * included) times the cold start's objective scaling sf; z = max(sf z, warm_mu / slack); mu = warm_mu,
+ * no least-squares multipliers.  The NLP scaling is the cold start's.  Returns -1 without solving where
+ * p->bound_value < 1e19 (the record has no state-bound multipliers) or where the cold start would scale a
+ * constraint row. */
+int mpc_oracle_solve_warm(const mpc_oracle_params *p, const double *state6, const double *coeffs, int ncoef,
+                          const ipm_options *opt, const double *warm_record, double warm_mu,
+                          double *u0, double *pred, double *sol, double *lambda, double *zl, double *zu,
+                          mpc_oracle_result *res);
+
 /* Pre-step (driving_state.cpp:196-235): waypoints (global frame) -> robot frame,
  * cubic least-squares fit by Householder QR, cte = c[0], etheta by the
  * reference's atan2 rule.  Returns 0 on success. */

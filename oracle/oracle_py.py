@@ -89,6 +89,9 @@ class Oracle:
         L.mpc_oracle_solve.restype = C.c_int
         L.mpc_oracle_solve.argtypes = [C.POINTER(OracleParams), _dp, _dp, C.c_int, C.POINTER(IpmOptions),
                                        _dp, _dp, _dp, _dp, _dp, _dp, C.POINTER(OracleResult)]
+        L.mpc_oracle_solve_warm.restype = C.c_int
+        L.mpc_oracle_solve_warm.argtypes = [C.POINTER(OracleParams), _dp, _dp, C.c_int, C.POINTER(IpmOptions), _dp,
+                                            C.c_double, _dp, _dp, _dp, _dp, _dp, _dp, C.POINTER(OracleResult)]
         L.mpc_oracle_eval_fg.argtypes = [C.POINTER(OracleParams), _dp, C.c_int, _dp, _dp, _dp]
         L.mpc_oracle_eval_grad.argtypes = [C.POINTER(OracleParams), _dp, C.c_int, _dp, _dp]
         L.mpc_oracle_eval_jac_dense.argtypes = [C.POINTER(OracleParams), _dp, C.c_int, _dp, _dp]
@@ -114,7 +117,9 @@ class Oracle:
         self.lib.ipm_default_options(C.byref(o))
         return o
 
-    def solve(self, pm, state, coeffs, opt=None):
+    def solve(self, pm, state, coeffs, opt=None, warm=None, warm_mu=1e-3):
+        """warm: a warm-start record (mpc_b200_warm_size(N) doubles, the GPU path's layout) or None for the cold start.
+        A warm solve needs BOUND >= 1e19 (no state bounds)."""
         p = params_from_map(pm)
         N = p.mpc_steps
         n, m = 8 * N - 2, 6 * N
@@ -122,9 +127,19 @@ class Oracle:
         u0 = np.zeros(2); pred = np.zeros(3 * N); sol = np.zeros(n); lam = np.zeros(m)
         zl = np.zeros(n); zu = np.zeros(n)
         r = OracleResult()
-        self.lib.mpc_oracle_solve(C.byref(p), _ptr(state), _ptr(coeffs), len(coeffs),
-                                  C.byref(opt) if opt is not None else None,
-                                  _ptr(u0), _ptr(pred), _ptr(sol), _ptr(lam), _ptr(zl), _ptr(zu), C.byref(r))
+        o = C.byref(opt) if opt is not None else None
+        if warm is None:
+            self.lib.mpc_oracle_solve(C.byref(p), _ptr(state), _ptr(coeffs), len(coeffs), o,
+                                      _ptr(u0), _ptr(pred), _ptr(sol), _ptr(lam), _ptr(zl), _ptr(zu), C.byref(r))
+        else:
+            warm = _arr(warm)
+            if warm.shape != (n + m + 4 * (N - 1),):
+                raise ValueError("warm record of %s doubles, expected %d" % (warm.shape, n + m + 4 * (N - 1)))
+            rc = self.lib.mpc_oracle_solve_warm(C.byref(p), _ptr(state), _ptr(coeffs), len(coeffs), o, _ptr(warm),
+                                                float(warm_mu), _ptr(u0), _ptr(pred), _ptr(sol), _ptr(lam), _ptr(zl),
+                                                _ptr(zu), C.byref(r))
+            if rc == -1:
+                raise ValueError("warm start refused: finite state bounds or a scaled constraint row")
         return dict(u0=u0, pred=pred.reshape(3, N), sol=sol, lam=lam, zl=zl, zu=zu, status=r.status,
                     iters=r.iters, obj=r.obj, kkt_error=r.kkt_error, dual_inf=r.dual_inf,
                     constr_viol=r.constr_viol, compl_inf=r.compl_inf,

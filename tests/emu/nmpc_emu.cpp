@@ -5,9 +5,11 @@
 // a problem in a lane and the write-out of its results) sequentially on the host, one emulated CTA of
 // PB lanes at a time.  What is the emulator's own is the driver: the kernel's cycle (nmpc_kernel.cuh)
 // as one loop per phase over the lanes and their stage groups of SPT stages, in the kernel's phase
-// order and in ascending groups, in place of the barriers; the P2 loop; and the counters.  (The
-// kernel's work queue is not emulated: lanes get their problems statically, and there is no warm-start
-// input; results do not depend on the lane, which the tests check.)  It exists so that the solver
+// order and in ascending groups, in place of the barriers; the P2 loop; the warm start's roll-out in P4
+// (control_loop's MODE_ROLLOUT branch); and the counters.  (The kernel's work queue is not emulated: lanes
+// get their problems statically; results do not depend on the lane, which the tests check.)  With a
+// warm-start record (warm_in) it runs the kernel's warm instantiation: lane_start<true> and
+// stages_init<SPT, true, ...>.  It exists so that the solver
 // LOGIC can be checked against the oracle in the CPU-only test tier (this container has no GPU).  It
 // is built only by tests/ into tests/emu/libnmpc_emu.so, is never linked into libmpc_b200.so, and
 // nothing in the product path can reach it.
@@ -27,7 +29,7 @@ static const int SPT = 2;   // same grouping of partial sums as the kernel's sta
 // The kernel's arguments for one batch.  prm14: dt, ref_cte, ref_etheta, ref_vel, w_cte, w_etheta, w_vel, w_angvel,
 // w_accel, max_angvel, max_throttle, w_angvel_d, w_accel_d, bound_value (0 = the 1e3 default).
 static SolveArgs emu_args(int N, const double *prm14, double tol, int max_iter, int PB, int batch, int ncoef,
-                          const double *state, const double *coeffs, const double *ref_vel,
+                          const double *state, const double *coeffs, const double *ref_vel, const double *warm_in, double warm_mu,
                           double *u0, double *pred, double *obj, int *status, int *iters, double *kkt, double *warm_out)
 {
     SolveArgs a = {};
@@ -37,7 +39,7 @@ static SolveArgs emu_args(int N, const double *prm14, double tol, int max_iter, 
     prm.w_cte = prm14[4]; prm.w_etheta = prm14[5]; prm.w_vel = prm14[6]; prm.w_angvel = prm14[7];
     prm.w_accel = prm14[8]; prm.max_angvel = prm14[9]; prm.max_throttle = prm14[10];
     prm.tol = tol; prm.max_iter = max_iter;
-    prm.warm_mu = 1e-3;
+    prm.warm_mu = warm_mu;
     prm.w_angvel_d = prm14[11]; prm.w_accel_d = prm14[12];
     prm.grp = SPT;
     prm.idt = 1.0 / prm.dt;
@@ -46,10 +48,11 @@ static SolveArgs emu_args(int N, const double *prm14, double tol, int max_iter, 
     a.PB = PB; a.batch = batch; a.ncoef = ncoef;
     a.state = state; a.coeffs = coeffs; a.ref_vel = ref_vel;
     a.u0 = u0; a.pred = pred; a.obj = obj; a.status = status; a.iters = iters; a.kkt = kkt; a.warm_out = warm_out;
+    a.warm_in = warm_in;
     return a;
 }
 
-template <bool RATE, int NC = 4>
+template <bool RATE, int NC = 4, bool WARM = false>
 static int emu_run(const SolveArgs &a, int *n_reg)
 {
     const Params &prm = a.prm;
@@ -75,7 +78,7 @@ static int emu_run(const SolveArgs &a, int *n_reg)
         // ---- "refill": every lane starts its problem
         for (int p = 0; p < np; p++) {
             sm.I(PI_NEXT, p) = base + p;
-            lane_start<false, NC>(prm, sm, ctrl[p], p, a, base + p, N, batch);
+            lane_start<WARM, NC>(prm, sm, ctrl[p], p, a, base + p, N, batch);
             nreg[p] = 0; for (int q = 0; q < 4; q++) g_kind_lane[4 * p + q] = 0;
         }
         for (;;) {
@@ -85,17 +88,27 @@ static int emu_run(const SolveArgs &a, int *n_reg)
             for (int p = 0; p < np; p++) g_lane_cycles += (sm.I(PI_MODE, p) != MODE_IDLE);
             // ---- P3a
             for (int p = 0; p < np; p++)
-                for (int g = 0; g < NG; g++) stages_init<SPT, false, RATE, NC>(prm, sm, RUN(p, g), a, N, batch);
+                for (int g = 0; g < NG; g++) stages_init<SPT, WARM, RATE, NC>(prm, sm, RUN(p, g), a, N, batch);
             for (int p = 0; p < np; p++) ctrl_handover(sm, p);
             // ---- P3b
             for (int p = 0; p < np; p++)
                 for (int g = 0; g < NG; g++) stages_coeffs<SPT, RATE, NC>(prm, sm, RUN(p, g), N);
             // ---- P4
-            for (int p = 0; p < np; p++)
+            for (int p = 0; p < np; p++) {
                 if (sm.I(PI_MODE, p) == MODE_NEWTON) {
                     sys[p] = ctrl_newton_backward<RATE>(prm, sm, p);
                     nreg[p] += ctrl_newton_forward<RATE>(prm, sm, ctrl[p], p, sys[p]);
                 }
+                if (WARM && sm.I(PI_MODE, p) == MODE_ROLLOUT) {
+                    // as control_loop: the roll-out of the warm controls, then a plain evaluation of the start point
+                    const size_t i = (size_t)sm.I(PI_PROB, p);
+                    double c4[NC];
+                    for (int q = 0; q < NC; q++) c4[q] = q < a.ncoef ? a.coeffs[(size_t)q * batch + i] : 0.0;
+                    ctrl_rollout<NC>(prm, sm, p, c4);
+                    sm.I(PI_MODE, p) = MODE_EVAL;
+                    sm.I(PI_FLAGS, p) = 0;
+                }
+            }
             // ---- P5
             for (int p = 0; p < np; p++)
                 for (int g = 0; g < NG; g++) {
@@ -154,12 +167,15 @@ extern "C" long long nmpc_emu_lane_cycles(int reset) { const long long v = g_lan
 extern "C" int nmpc_emu_solve(int N, const double *prm14, double tol, int max_iter, int PB, int batch,
                               const double *state, const double *coeffs, const double *ref_vel,
                               double *u0, double *pred, double *obj, int *status, int *iters, double *kkt,
-                              double *warm_out /* warm_size x batch, optional */, int *n_reg /* batch, optional */)
+                              double *warm_out /* warm_size x batch, optional */, int *n_reg /* batch, optional */,
+                              const double *warm_in /* warm_size x batch, NULL = cold start */, double warm_mu)
 {
-    const SolveArgs a = emu_args(N, prm14, tol, max_iter, PB, batch, 4, state, coeffs, ref_vel, u0, pred, obj, status, iters, kkt,
-                                 warm_out);
+    const SolveArgs a = emu_args(N, prm14, tol, max_iter, PB, batch, 4, state, coeffs, ref_vel, warm_in, warm_mu, u0, pred, obj,
+                                 status, iters, kkt, warm_out);
     // prm14[11], prm14[12]: w_angvel_d, w_accel_d (rate penalties) select the augmented-Riccati variant
-    if (prm14[11] != 0.0 || prm14[12] != 0.0) return emu_run<true>(a, n_reg);
+    const bool rate = prm14[11] != 0.0 || prm14[12] != 0.0;
+    if (warm_in) return rate ? emu_run<true, 4, true>(a, n_reg) : emu_run<false, 4, true>(a, n_reg);
+    if (rate) return emu_run<true>(a, n_reg);
     return emu_run<false>(a, n_reg);
 }
 
@@ -167,11 +183,14 @@ extern "C" int nmpc_emu_solve(int N, const double *prm14, double tol, int max_it
 // kernel uses for orders above 3.
 extern "C" int nmpc_emu_solve_poly(int N, const double *prm14, double tol, int max_iter, int PB, int batch, int ncoef,
                                    const double *state, const double *coeffs, double *u0, double *pred, double *obj,
-                                   int *status, int *iters, double *kkt)
+                                   int *status, int *iters, double *kkt, double *warm_out /* optional */,
+                                   const double *warm_in /* NULL = cold start */, double warm_mu)
 {
     if (ncoef < 4 || ncoef > NMPC_MAX_COEFFS) return -1;
-    const SolveArgs a = emu_args(N, prm14, tol, max_iter, PB, batch, ncoef, state, coeffs, nullptr, u0, pred, obj, status, iters,
-                                 kkt, nullptr);
-    if (prm14[11] != 0.0 || prm14[12] != 0.0) return emu_run<true, NMPC_MAX_COEFFS>(a, nullptr);
+    const SolveArgs a = emu_args(N, prm14, tol, max_iter, PB, batch, ncoef, state, coeffs, nullptr, warm_in, warm_mu, u0, pred, obj,
+                                 status, iters, kkt, warm_out);
+    const bool rate = prm14[11] != 0.0 || prm14[12] != 0.0;
+    if (warm_in) return rate ? emu_run<true, NMPC_MAX_COEFFS, true>(a, nullptr) : emu_run<false, NMPC_MAX_COEFFS, true>(a, nullptr);
+    if (rate) return emu_run<true, NMPC_MAX_COEFFS>(a, nullptr);
     return emu_run<false, NMPC_MAX_COEFFS>(a, nullptr);
 }

@@ -17,15 +17,17 @@ MAX_ITER = 100
 
 
 def _oracle_chunk(args):
+    """args: (pm, state, coeffs) or (pm, state, coeffs, warm records, warm_mu) for warm-started solves"""
     from oracle.oracle_py import Oracle
-    pm, state, coeffs = args
+    pm, state, coeffs = args[:3]
+    warm, warm_mu = args[3:] if len(args) > 3 else (None, 1e-3)
     orc = Oracle()
     opt = orc.default_options(); opt.max_iter = MAX_ITER
     B = state.shape[1]
     out = dict(u0=np.zeros((2, B)), obj=np.zeros(B), status=np.zeros(B, dtype=np.int32), iters=np.zeros(B, dtype=np.int32),
                kkt=np.zeros(B))
     for i in range(B):
-        r = orc.solve(pm, state[:, i], coeffs[:, i], opt)
+        r = orc.solve(pm, state[:, i], coeffs[:, i], opt, warm=None if warm is None else warm[:, i], warm_mu=warm_mu)
         out["u0"][:, i] = r["u0"]; out["obj"][i] = r["obj"]; out["status"][i] = r["status"]
         out["iters"][i] = r["iters"]; out["kkt"][i] = r["kkt_error"]
     return out

@@ -13,7 +13,8 @@ from tests.problems import mild, generated, restoration_cases
 _EMU = None
 
 
-def emu_solve(pm, state, coeffs, PB=4, tol=1e-8, max_iter=200, ref_vel=None):
+def emu_solve(pm, state, coeffs, PB=4, tol=1e-8, max_iter=200, ref_vel=None, warm=None, warm_mu=1e-3):
+    """warm: warm-start records (warm_size x B, the kernel's layout) or None for the cold start."""
     global _EMU
     if _EMU is None:
         _EMU = C.CDLL(os.path.join(os.path.dirname(os.path.abspath(__file__)), "emu", "libnmpc_emu.so"))
@@ -25,15 +26,18 @@ def emu_solve(pm, state, coeffs, PB=4, tol=1e-8, max_iter=200, ref_vel=None):
                    dtype=np.float64)
     state = np.ascontiguousarray(state, dtype=np.float64); coeffs = np.ascontiguousarray(coeffs, dtype=np.float64)
     u0 = np.zeros((2, B)); pred = np.zeros((3 * N, B)); obj = np.zeros(B); kkt = np.zeros(B)
-    warm = np.zeros((capi.lib().mpc_b200_warm_size(N), B))     # the kernel's warm-start record
+    rec = np.zeros((capi.lib().mpc_b200_warm_size(N), B))      # the kernel's warm-start record
     st = np.zeros(B, dtype=np.int32); it = np.zeros(B, dtype=np.int32); nreg = np.zeros(B, dtype=np.int32)
     rv = None if ref_vel is None else np.ascontiguousarray(ref_vel, dtype=np.float64).ctypes.data_as(dp)
     P = lambda a: a.ctypes.data_as(dp)  # noqa: E731
+    if warm is not None:
+        warm_in = np.ascontiguousarray(warm, dtype=np.float64)
+        assert warm_in.shape == warm.shape == (capi.lib().mpc_b200_warm_size(N), B)
     _EMU.nmpc_emu_solve(C.c_int(N), P(prm), C.c_double(tol), C.c_int(max_iter), C.c_int(PB), C.c_int(B), P(state),
                         P(coeffs), rv, P(u0), P(pred), P(obj), st.ctypes.data_as(ip), it.ctypes.data_as(ip), P(kkt),
-                        P(warm), nreg.ctypes.data_as(ip))
+                        P(rec), nreg.ctypes.data_as(ip), None if warm is None else P(warm_in), C.c_double(warm_mu))
     n = 8 * N - 2       # equality multipliers: rows [n, n + 6N) of the record
-    return dict(u0=u0, pred=pred, obj=obj, status=st, iters=it, kkt=kkt, lam=warm[n:n + 6 * N], warm=warm, nreg=nreg)
+    return dict(u0=u0, pred=pred, obj=obj, status=st, iters=it, kkt=kkt, lam=rec[n:n + 6 * N], warm=rec, nreg=nreg)
 
 
 def test_emu_matches_oracle_mild(oracle):
@@ -173,7 +177,7 @@ def test_emu_small_weights_keep_lsq_multipliers(oracle):
     assert kept == 16      # (the converged multipliers are small too: the start was not the discarded kind)
 
 
-def emu_solve_poly(pm, state, coeffs, PB=4, tol=1e-8, max_iter=200):
+def emu_solve_poly(pm, state, coeffs, PB=4, tol=1e-8, max_iter=200, warm=None, warm_mu=1e-3):
     """Path polynomial of order coeffs.shape[0] - 1 in 4..7 (the kernel's higher-order instantiation)."""
     emu_solve(pm, state[:, :1], coeffs[:4, :1])      # (loads the library)
     dp = C.POINTER(C.c_double); ip = C.POINTER(C.c_int)
@@ -185,11 +189,16 @@ def emu_solve_poly(pm, state, coeffs, PB=4, tol=1e-8, max_iter=200):
     state = np.ascontiguousarray(state, dtype=np.float64); coeffs = np.ascontiguousarray(coeffs, dtype=np.float64)
     u0 = np.zeros((2, B)); pred = np.zeros((3 * N, B)); obj = np.zeros(B); kkt = np.zeros(B)
     st = np.zeros(B, dtype=np.int32); it = np.zeros(B, dtype=np.int32)
+    rec = np.zeros((capi.lib().mpc_b200_warm_size(N), B))
     P = lambda a: a.ctypes.data_as(dp)  # noqa: E731
+    if warm is not None:
+        warm_in = np.ascontiguousarray(warm, dtype=np.float64)
+        assert warm_in.shape == rec.shape
     rc = _EMU.nmpc_emu_solve_poly(C.c_int(N), P(prm), C.c_double(tol), C.c_int(max_iter), C.c_int(PB), C.c_int(B), C.c_int(nc),
-                                  P(state), P(coeffs), P(u0), P(pred), P(obj), st.ctypes.data_as(ip), it.ctypes.data_as(ip), P(kkt))
+                                  P(state), P(coeffs), P(u0), P(pred), P(obj), st.ctypes.data_as(ip), it.ctypes.data_as(ip), P(kkt),
+                                  P(rec), None if warm is None else P(warm_in), C.c_double(warm_mu))
     assert rc == 0
-    return dict(u0=u0, pred=pred, obj=obj, status=st, iters=it, kkt=kkt)
+    return dict(u0=u0, pred=pred, obj=obj, status=st, iters=it, kkt=kkt, warm=rec)
 
 
 def higher_order(seed, batch, ncoef):

@@ -859,7 +859,8 @@ def test_state_bounds_honoured_or_refused(oracle, bound):
     assert n_inside + n_flag == 64
 
 
-def _oracle_many(pm, state, coeffs, max_iter=100):
+def _oracle_many(pm, state, coeffs, max_iter=100, warm=None, warm_mu=1e-3):
+    """the oracle on all host cores; warm: warm-start records (warm_size x B) or None for cold starts"""
     import multiprocessing as mp
     from tests.parity_sweep import _oracle_chunk
     import tests.parity_sweep as ps
@@ -867,8 +868,10 @@ def _oracle_many(pm, state, coeffs, max_iter=100):
     n = state.shape[1]
     P = os.cpu_count() or 1
     cuts = np.linspace(0, n, 4 * P + 1).astype(int)
+    w = (lambda a, b: ()) if warm is None else (lambda a, b: (warm[:, a:b].copy(), warm_mu))  # noqa: E731
     with mp.get_context("fork").Pool(P) as pool:
-        parts = pool.map(_oracle_chunk, [(pm, state[:, a:b].copy(), coeffs[:, a:b].copy()) for a, b in zip(cuts[:-1], cuts[1:]) if b > a])
+        parts = pool.map(_oracle_chunk, [(pm, state[:, a:b].copy(), coeffs[:, a:b].copy()) + w(a, b)
+                                         for a, b in zip(cuts[:-1], cuts[1:]) if b > a])
     return {k: np.concatenate([p[k] for p in parts], axis=-1) for k in parts[0]}
 
 
@@ -974,17 +977,35 @@ def test_packed_and_sliced_ticks_equal_the_plain_tick():
 
 
 def test_host_warm_records_are_staged(oracle):
-    """SURVEY 8b ownership: warm-start records may live in host memory too."""
+    """SURVEY 8b ownership: warm-start records may live in host memory too.  Host and device records give the same solves
+    bit for bit: u0, pred, iterations, status and the records written, cold and warm."""
+    torch = pytest.importorskip("torch")
+    dev = torch.device("cuda:0")
     state, coeffs = mild(7, 16)
+    state2 = state.copy(); state2[3] += 0.02; state2[4] -= 0.01
     sv = _solver(YAML_DEFAULT, 16)
     N = 20; ws = capi.lib().mpc_b200_warm_size(N)
-    w = np.zeros((ws, 16))
-    out = dict(u0=np.zeros((2, 16)), pred=np.zeros((3 * N, 16)), status=np.zeros(16, dtype=np.int32), iters=np.zeros(16, dtype=np.int32))
-    sv.solve_raw(16, state, coeffs, out["u0"], out["pred"], status=out["status"], iters=out["iters"], warm_out=w)
-    assert np.all(out["status"] == 1) and np.abs(w).max() > 0
-    out2 = dict(u0=np.zeros((2, 16)), pred=np.zeros((3 * N, 16)), status=np.zeros(16, dtype=np.int32), iters=np.zeros(16, dtype=np.int32))
-    sv.solve_raw(16, state, coeffs, out2["u0"], out2["pred"], status=out2["status"], iters=out2["iters"], warm_in=w)
+
+    def run(on_dev, st, warm_in):
+        """one solve with the records in host (on_dev False) or device memory; inputs and other outputs on the host"""
+        out = dict(u0=np.zeros((2, 16)), pred=np.zeros((3 * N, 16)), status=np.zeros(16, dtype=np.int32),
+                   iters=np.zeros(16, dtype=np.int32))
+        wo = torch.zeros((ws, 16), dtype=torch.float64, device=dev) if on_dev else np.zeros((ws, 16))
+        wi = None if warm_in is None else (torch.from_numpy(warm_in).to(dev) if on_dev else warm_in.copy())
+        sv.solve_raw(16, st, coeffs, out["u0"], out["pred"], status=out["status"], iters=out["iters"], warm_in=wi, warm_out=wo)
+        out["rec"] = wo.cpu().numpy() if on_dev else wo
+        return out
+
+    res = {}
+    for on_dev in (False, True):
+        cold = run(on_dev, state, None)
+        res[on_dev] = (cold, run(on_dev, state, cold["rec"]), run(on_dev, state2, cold["rec"]))
     sv.close()
-    assert np.all(out2["status"] == 1)
-    assert np.abs(out2["u0"] - out["u0"]).max() <= U_TOL
-    assert out2["iters"].mean() < out["iters"].mean()
+    cold, same, moved = res[False]
+    assert np.all(cold["status"] == 1) and np.abs(cold["rec"]).max() > 0
+    assert np.all(same["status"] == 1) and np.all(moved["status"] == 1)
+    assert np.abs(same["u0"] - cold["u0"]).max() <= U_TOL
+    assert same["iters"].mean() < cold["iters"].mean()
+    for h, d in zip(res[False], res[True]):
+        for k in ("u0", "pred", "status", "iters", "rec"):
+            assert h[k].tobytes() == d[k].tobytes(), k

@@ -51,6 +51,7 @@ ROWS += [
     ("N100-cold", YAML_DEFAULT, 100, 12, {}, False, 6, _k(2, 6, False, False)),
     ("N100-warm", YAML_DEFAULT, 100, 12, {}, True, 6, _k(2, 0, True, False)),
     ("nc6-cold", YAML_DEFAULT, 20, 4, {"poly_coeffs": 6}, False, 4, _k(2, 0, False, False, 8)),
+    ("nc6-warm", YAML_DEFAULT, 20, 4, {"poly_coeffs": 6}, True, 4, _k(2, 0, True, False, 8)),
     ("nc6-rate-warm", CFG_DEFAULT, 20, 4, {"poly_coeffs": 6}, True, 4, _k(2, 0, True, True, 8)),
     ("pb7", YAML_DEFAULT, 20, 14, {"problems_per_cta": 7}, False, 7, _k(2, 0, False, False)),
 ]
